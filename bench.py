@@ -8,7 +8,9 @@ launched from libmtdgan_sm100a.so.  Also reports generator inference on 1x512x51
 Reference arm (`--impl reference`): the CPU oracle port of the same step on the box's host cores (the Python
 reference cannot travel to the GPU box; SURVEY §8c).
 
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  `--dump-outputs DIR` also writes what the last timed train step computed (losses,
+loss terms, the weights it leaves) as DIR/<name>.npy.  Every timed step starts from the same seeded state on the same
+inputs, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -46,6 +48,7 @@ def emit(line: dict):
         os.write(_JSON_FD, (json.dumps(line) + "\n").encode())
 
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 PATCH, BATCH = 64, 20
@@ -141,6 +144,28 @@ GROUPS = {"conv": ("mtd_conv_fwd", "mtd_conv_fwd_tc", "mtd_conv_dgrad", "mtd_con
           "spectral_norm": ("mtd_sn_power_iter",), "pcgrad": ("mtd_pcgrad_project",), "adamw": ("mtd_adamw_step",)}
 
 
+DUMP_D_SAMPLE = 1 << 20      # discriminator parameters --dump-outputs writes: a fixed, seeded sample of the 68.4 M
+
+
+def step_outputs(out, model):
+    """What a train step hands its caller, as float32 host arrays: the losses and loss terms it returns and the weights
+    it leaves behind (every generator parameter, DUMP_D_SAMPLE discriminator parameters at seeded positions)."""
+    d_losses, d_det, g_loss, g_det = out
+    arrays = {"d_losses": d_losses, "g_loss": g_loss}
+    arrays.update({k.replace("/", "_"): v for k, v in {**d_det, **g_det}.items()})       # 'D/real_enc' -> D_real_enc
+    arrays["generator_params"] = torch.cat([p.detach().flatten() for p in model.Generator.parameters()])
+    d_flat = torch.cat([p.detach().flatten() for p in model.Discriminator.parameters()])
+    idx = torch.randint(0, d_flat.numel(), (DUMP_D_SAMPLE,), generator=torch.Generator().manual_seed(0))
+    arrays["discriminator_params_sample"] = d_flat[idx.to(d_flat.device)]
+    return {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_own(args):
     import mtdgan_b200
     from mtdgan_b200 import _ext
@@ -173,6 +198,11 @@ def run_own(args):
     gparams = list(G.parameters())
     runner = GraphedTrainStep(model, opt_D, opt_G, wm,
                               post_g_backward=(lambda: mdist.allreduce_mean_grads(gparams)) if world > 1 else None)
+    # Every timed step starts from this state (weights, spectral-norm vectors, optimizer moments, RNGs), restored outside
+    # the timed window.  The fp32 atomics of some kernels differ in the last bits from run to run, and the GAN's
+    # trajectory grows such differences to O(1) within a few dozen steps: a fixed start keeps each step's outputs
+    # reproducible, and the work a step does does not depend on the values.
+    init_state = runner._snapshot()
 
     def eager_step(x, y):
         dl, _, gl, _ = runner.eager_step(x, y)
@@ -192,8 +222,11 @@ def run_own(args):
         else:
             runner.capture(xd, yd, warmup=2)
 
+    last = [None]             # what the latest step returned (graph output buffers: valid until the next replay)
+
     def step(x, y):
-        dl, _, gl, _ = runner(x, y)
+        last[0] = runner(x, y)
+        dl, _, gl, _ = last[0]
         return dl, gl
 
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)      # > 126 MB L2
@@ -207,6 +240,7 @@ def run_own(args):
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n)]
         sink = torch.empty(4, dtype=torch.float32).pin_memory()
         for s, e in ev:
+            runner._restore(init_state)
             flush.zero_()
             s.record()
             if e2e:
@@ -231,6 +265,8 @@ def run_own(args):
     ms_e2e = timed(args.steps, e2e=True)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, step_outputs(last[0], model))
     t_dev, t_e2e = sum(ms), sum(ms_e2e)
     if world > 1:
         t = torch.tensor([t_dev, t_e2e], device=dev, dtype=torch.float64)
@@ -369,6 +405,8 @@ def run_own(args):
                                "(BASELINE configs[2]/[3])", "global_batch": patches, "patch": PATCH,
                    "parallelism": f"dp{world}", "l2": "256 MiB buffer written between timed steps (L2 flush)",
                    "weights": "random init, seed 2024", "optimizer": "fused AdamW lr 1e-4 wd 5e-4",
+                   "timed_step_state": "every timed step starts from the seeded initial weights, optimizer state and RNGs "
+                                       "(restored outside the timed window)",
                    "execution": "whole step replayed as one CUDA graph" if use_graph else "eager launches",
                    "conv_precision": "tcgen05 3xTF32 (fp32-grade) + exact fp32 SIMT for thin/strided layers"},
         "e2e": {"value": round(patches * args.steps / (t_e2e * 1e-3), 3), "unit": "patches/s",
@@ -645,35 +683,25 @@ def run_reference(args):
     from oracle.mtdgan_oracle import synthetic_pair
     torch.set_num_threads(os.cpu_count())
     tr = OracleTrainer(oracle_state())
-    # The batch is ALWAYS the GPU arm's (20 patches): the ratio the driver computes must compare equal configurations.
-    # What is bounded on a slow host is the NUMBER of timed steps (patches/s is a rate): the first step calibrates, and
-    # the run is cut to what fits ~4 minutes -- never below 2 timed steps -- and says so in `cpu_baseline.sample`.
+    # The batch is ALWAYS the GPU arm's (20 patches), so the two arms compare equal configurations; --steps sets the
+    # number of timed steps (patches/s is a rate, so fewer steps suit a slow host).  At least one untimed step runs first.
     batch = BATCH
     x, y = synthetic_pair(batch, PATCH, seed=1234)
-    t0 = time.perf_counter(); tr.step(x, y); t_cal = time.perf_counter() - t0
-    warm = max(0, args.warmup - 1)
-    timed_steps = args.steps
-    if t_cal * (args.steps + warm) > 240.0:
-        warm = 0
-        timed_steps = max(2, min(args.steps, int(240.0 / t_cal)))
-        print(f"[bench --impl reference] host too slow for {args.steps} steps of B={batch} ({t_cal:.1f} s/step): "
-              f"timing {timed_steps} steps", file=sys.stderr)
-    for _ in range(warm):
+    for _ in range(max(1, args.warmup)):
         tr.step(x, y)
     t0 = time.perf_counter()
-    for _ in range(timed_steps):
+    for _ in range(args.steps):
         tr.step(x, y)
     dt = time.perf_counter() - t0
-    v = round(batch * timed_steps / dt, 4)
+    v = round(batch * args.steps / dt, 4)
     return {"impl": "reference", "metric": "train patches/s (64x64, bs20/GPU)", "value": v, "unit": "patches/s", "n_gpus": args.gpus,
-            "steps": args.steps, "warmup": args.warmup, "ms_per_step": round(dt / timed_steps * 1e3, 2), "higher_is_better": True,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": round(dt / args.steps * 1e3, 2), "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": "MTD_GAN_Method full train step (G + MTL-D + RC/NDS + PCGrad + AdamW), 20 synthetic 1x64x64 "
                                    "patches (BASELINE configs[2]): CPU oracle port of the reference (torch-CPU, all host threads)",
                        "global_batch": batch, "patch": PATCH, "parallelism": "cpu"},
             "cpu_baseline": {"value": v, "unit": "patches/s", "cores": os.cpu_count(), "kind": "port",
-                             "sample": f"{timed_steps} timed steps of {batch} synthetic 64x64 patches each"
-                                       + ("" if timed_steps == args.steps else f" (cut from {args.steps}: slow host)")},
+                             "sample": f"{args.steps} timed steps of {batch} synthetic 64x64 patches each"},
             "e2e": {"value": v, "unit": "patches/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
 
 
@@ -687,7 +715,10 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of the captured CUDA graph")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the torch-eager-on-GPU baseline leg")
     ap.add_argument("--infer-batch", type=int, default=64, help="512x512 slices per GPU of the batched inference leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed train step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     claim_stdout()
     if args.impl == "reference":
         line = run_reference(args)

@@ -1,22 +1,22 @@
-"""Loads the LIVE reference (babbu3682/MTD-GAN) from /root/reference for oracle validation and
-golden-vector generation.  Only usable in the build container; GPU-box tests never call this."""
+"""Loads the LIVE reference (babbu3682/MTD-GAN) from the checkout named by $MTDGAN_REFERENCE, for regenerating
+the golden vectors under tests/golden/.  The tests never import the reference: they compare against those vectors."""
 import os
 import sys
 import types
 import importlib
 
-REF_ROOT = "/root/reference"
+REF_ROOT = os.environ.get("MTDGAN_REFERENCE", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF_ROOT, "arch", "Ours", "networks.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_ROOT, "arch", "Ours", "networks.py"))
 
 
 def load_reference():
     """Returns a namespace with the reference's hot-path modules.  The reference's top-level module
     names (losses, arch, module) collide with this repo's drop-in mirrors, so the reference is
     imported under a temporarily swapped sys.path / sys.modules and handed back as objects."""
-    assert reference_available()
+    assert reference_available(), "set MTDGAN_REFERENCE to a checkout of babbu3682/MTD-GAN"
     try:                       # the reference's losses.py imports torchvision; its op registration inspects sys.modules
         import torchvision  # noqa: F401   and must not run while the reference's namespace packages are half-imported
     except Exception:

@@ -1,7 +1,7 @@
-"""Generates the golden fixtures under tests/golden/ from the LIVE reference (/root/reference), on CPU.
+"""Generates the golden fixtures under tests/golden/ from the LIVE reference, on CPU.
 
-Run in the build container:   CUDA_VISIBLE_DEVICES="" python tests/golden/make_golden.py
-The fixtures travel with the repo; /root/reference does not exist on the GPU box.
+Run:   MTDGAN_REFERENCE=<checkout of babbu3682/MTD-GAN> CUDA_VISIBLE_DEVICES="" python tests/golden/make_golden.py
+The fixtures travel with the repo, so the tests need no copy of the reference.
 """
 import os
 import random
@@ -13,7 +13,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 import torch  # noqa: E402
 
-from _golden_util import GOLDEN_DIR, summarize  # noqa: E402
+from _golden_util import save, summarize  # noqa: E402
 from _refload import load_reference  # noqa: E402
 from oracle import mtdgan_oracle as O  # noqa: E402
 
@@ -36,11 +36,6 @@ class MaskDrop(torch.nn.Module):
 def drop_mask(b, seed):
     g = torch.Generator().manual_seed(seed)
     return (torch.rand(b, 512, generator=g) >= 0.3).float() / 0.7
-
-
-def save(name, obj):
-    torch.save(obj, os.path.join(GOLDEN_DIR, name))
-    print(f"wrote {name}: {os.path.getsize(os.path.join(GOLDEN_DIR, name)) / 1024:.1f} KiB")
 
 
 def seeded_model():
@@ -69,8 +64,8 @@ xb = (0.5 * torch.randn(1, 32, 64, 64, generator=g)).requires_grad_(True)
 wgt = torch.randn(1, 32, 64, 64, generator=g)
 out = blk(xb)
 (out * wgt).sum().backward()
-save("fftblock_64.pt", {"out": out.detach(), "dx": xb.grad,
-                        "grads": {k: p.grad.clone() for k, p in blk.named_parameters()}})
+save("fftblock_64.pt", {"out": out.detach(), "grads": {k: p.grad.clone() for k, p in blk.named_parameters()}})
+save("fftblock_64_dx.pt", {"dx": xb.grad})                       # a file of its own: each stays under 1 MB
 
 # 5. discriminator: train-mode forward/backward with an injected dropout mask, then eval ----------
 m = seeded_model()

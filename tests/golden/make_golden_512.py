@@ -1,6 +1,6 @@
-"""Regenerates tests/golden/gen_fwd_512.pt alone (fp32, 1 MiB) from the LIVE reference on CPU — the same statement
+"""Regenerates tests/golden/gen_fwd_512.pt alone (fp32) from the LIVE reference on CPU — the same statement
 as section 2/3 of make_golden.py, for when only this fixture changes.
-Run in the build container:   CUDA_VISIBLE_DEVICES="" python tests/golden/make_golden_512.py"""
+Run:   MTDGAN_REFERENCE=<checkout of babbu3682/MTD-GAN> CUDA_VISIBLE_DEVICES="" python tests/golden/make_golden_512.py"""
 import os
 import random
 import sys
@@ -11,7 +11,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 import torch  # noqa: E402
 
-from _golden_util import GOLDEN_DIR  # noqa: E402
+from _golden_util import save  # noqa: E402
 from _refload import load_reference  # noqa: E402
 from oracle import mtdgan_oracle as O  # noqa: E402
 
@@ -22,5 +22,4 @@ random.seed(2024)
 m = N.MTD_GAN_Method().eval()
 with torch.no_grad():
     out = m.Generator(O.synthetic_pair(1, 512, seed=12)[0])
-torch.save({"out": out}, os.path.join(GOLDEN_DIR, "gen_fwd_512.pt"))
-print("wrote gen_fwd_512.pt", tuple(out.shape), out.dtype)
+save("gen_fwd_512.pt", {"out": out})

@@ -1,7 +1,8 @@
 """Golden fixtures for the ablation rows (SURVEY §8f-3) from the LIVE reference on CPU: for each of the ten
 `Ablation_*` classes (arch/Ours/networks.py:1324-1936) the initial-state fingerprint, `d_loss` / `g_loss` totals and
 details on 2 synthetic patches with injected dropout masks, and fingerprints of the gradients `d_loss.backward()` /
-`g_loss.backward()` leave (engine.py:58-73).  Run:  CUDA_VISIBLE_DEVICES="" python tests/golden/make_golden_ablation.py"""
+`g_loss.backward()` leave (engine.py:58-73).
+Run:  MTDGAN_REFERENCE=<checkout of babbu3682/MTD-GAN> CUDA_VISIBLE_DEVICES="" python tests/golden/make_golden_ablation.py"""
 import contextlib
 import io
 import os
@@ -14,7 +15,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 import torch  # noqa: E402
 
-from _golden_util import GOLDEN_DIR, summarize  # noqa: E402
+from _golden_util import save, summarize  # noqa: E402
 from _refload import load_reference  # noqa: E402
 from oracle import mtdgan_oracle as O  # noqa: E402
 
@@ -101,5 +102,4 @@ torch.manual_seed(2024)
 G = N.REDCNN_Generator(in_channels=1, out_channels=32, num_layers=10, kernel_size=3, padding=1).eval()
 with torch.no_grad():
     out["redcnn_fwd_64"] = G(O.synthetic_pair(2, 64, seed=11)[0])
-torch.save(out, os.path.join(GOLDEN_DIR, "ablation.pt"))
-print("wrote ablation.pt", os.path.getsize(os.path.join(GOLDEN_DIR, "ablation.pt")) // 1024, "KiB")
+save("ablation.pt", out)

@@ -1,8 +1,7 @@
 """Data edge (SURVEY §8f-4): the GPU `window_patch` sampler against the numpy restatement of the reference's MONAI
-transform chain (create_datasets/Mayo.py:117-136), BIT-EXACT (byte / index work), and the checkpoint round trip with a
-state_dict written by the live reference (train.py:146-159, 276-288)."""
+transform chain (create_datasets/Mayo.py:117-136), BIT-EXACT (byte / index work), and the checkpoint round trip in the
+reference's checkpoint layout (train.py:146-159, 276-288)."""
 import io
-import os
 import random
 
 import numpy as np
@@ -114,23 +113,23 @@ def test_checkpoint_self_round_trip_cpu():
         assert torch.equal(a, b), k
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/arch/Ours/networks.py"), reason="needs the live reference")
-def test_checkpoint_written_by_reference_loads_and_returns():
-    """A checkpoint the REFERENCE writes (its MTD_GAN_Method + torch.optim.AdamW after one real CPU step, dict layout of
+def test_checkpoint_in_reference_layout_loads_and_returns():
+    """A checkpoint as the reference's train.py writes it (the model's state_dict under the reference's 326 keys, pinned
+    by its init fingerprint state_summary.pt; torch.optim.AdamW state after one optimizer step; dict layout of
     train.py:279-287, with DataParallel-style '.module' keys to exercise :149) loads into the drop-in model and the fused
-    optimizer, and a checkpoint the drop-in writes loads back into the reference classes — all tensors equal."""
-    from _refload import load_reference
+    optimizer, and a checkpoint the drop-in writes loads back into a model and torch.optim.AdamW — all tensors equal."""
+    from _golden_util import load
     from arch.Ours.networks import MTD_GAN_Method
     from mtdgan_b200 import checkpoint as CK
     from mtdgan_b200.optim import FusedAdamW
-    from oracle import mtdgan_oracle as O
-    ref = load_reference()
     torch.manual_seed(3); random.seed(3)
-    rm = ref.networks.MTD_GAN_Method()
+    rm = MTD_GAN_Method()
+    assert list(rm.state_dict().keys()) == list(load("state_summary.pt").keys())
     rD = torch.optim.AdamW([{"params": list(rm.Discriminator.parameters())}, {"params": [], "lr": 0.025}], lr=1e-4, weight_decay=5e-4)
     rG = torch.optim.AdamW(rm.Generator.parameters(), lr=1e-4, weight_decay=5e-4)
-    x, y = O.synthetic_pair(1, 64, seed=2)
-    rm.g_loss(x, y)[0].backward()                           # populates G grads and (dead) D grads: one real optimizer step each
+    g = torch.Generator().manual_seed(2)
+    for p in rm.parameters():                               # seeded gradients (the drop-in has no CPU forward): one step each
+        p.grad = 1e-3 * torch.randn(p.shape, generator=g)
     rD.step(); rG.step()
     sch = torch.optim.lr_scheduler.LambdaLR(rG, lambda e: 0.5)
     ck = {"model_state_dict": {k.replace("Generator.", "Generator.module.", 1) if k.startswith("Generator.encoder.0") else k: v
@@ -146,11 +145,14 @@ def test_checkpoint_written_by_reference_loads_and_returns():
     for rp, mp in zip(rm.Generator.parameters(), mine.Generator.parameters()):
         for key in ("step", "exp_avg", "exp_avg_sq"):
             assert torch.equal(torch.as_tensor(rG.state[rp][key]).float(), torch.as_tensor(mG.state[mp][key]).float().cpu()), key
-    # and back: what the drop-in writes, the reference classes load
+    # and back: what the drop-in writes, a fresh model and torch.optim.AdamW load
     back = CK.checkpoint_dict(mine, mD, None, mG, None, epoch=5)
-    rm2 = ref.networks.MTD_GAN_Method()
+    rm2 = MTD_GAN_Method()
     rm2.load_state_dict(back["model_state_dict"])
     rG2 = torch.optim.AdamW(rm2.Generator.parameters(), lr=1e-4, weight_decay=5e-4)
     rG2.load_state_dict(back["optimizer_G"])
     for (k, a), (_, b) in zip(rm.state_dict().items(), rm2.state_dict().items()):
         assert torch.equal(a, b), k
+    for rp, rp2 in zip(rm.Generator.parameters(), rm2.Generator.parameters()):
+        for key in ("step", "exp_avg", "exp_avg_sq"):
+            assert torch.equal(torch.as_tensor(rG.state[rp][key]).float(), torch.as_tensor(rG2.state[rp2][key]).float()), key
