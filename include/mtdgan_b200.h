@@ -99,6 +99,14 @@ int mtd_conv_wgrad_finish(const float* gp, float* dw_ref, int transposed, int Co
  * pre-scaled, 4 = correction-only instance without a gp).                                                  */
 int mtd_act_bwd_sn(const float* dy, const float* y, float* dz, float* dbias, const float* bias, double* zw,
                    const float* dz_scale, int groups, long long M, int N, int act, float slope, void* stream);
+/* mtd_act_bwd of one backward pass that also folds its dz into accumulators spanning several passes over the same
+ * forward graph (the gradient of a sum of losses is linear in dz): dz (optional, unscaled, as mtd_act_bwd writes it);
+ * acc[M][N] = (acc_first ? 0 : acc) + dz * inv_sigma[g] (inv_sigma optional: scale 1); dbias (optional) += column sums
+ * of dz; zw (optional, as mtd_act_bwd_sn: act none or leaky) += per-call sums of dz . (y_pre - bias).  The batch
+ * holds `groups` (<= 4) calls of M/groups rows.  y may be null when act is none and zw is null.  dbias and zw are
+ * accumulated (zero them before the first pass).  Any N <= 8192.                                             */
+int mtd_act_bwd_acc(const float* dy, const float* y, float* dz, float* acc, int acc_first, float* dbias, const float* bias,
+                    double* zw, const float* inv_sigma, int groups, long long M, int N, int act, float slope, void* stream);
 /* elements per chunk-table entry of a segment with kh*kw = taps and Cin = cin: a whole number of packed rows when a
  * row fits the kernels' shared-memory staging (coalesced transposition), else a fixed block                     */
 int mtd_wgrad_finish_chunk_elems(int taps, int cin);

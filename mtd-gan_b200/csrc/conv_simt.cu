@@ -1179,8 +1179,21 @@ int launch_wgrad(WgradArgs& a, cudaStream_t st) {
 // dz = dy * act'(y)  (+ per-channel sums of dz accumulated into dbias, pre-zeroed by the caller
 // wrapper).  (M, N) row-major, N = channels.
 // ---------------------------------------------------------------------------------------------
+// Fold outputs of mtd_act_bwd_acc (the FOLD instantiations below): dz of one backward pass is also folded into an
+// accumulator that spans several passes, acc (+)= dz * scale[g], with zw[g] += sum dz . (y_pre - bias) per batched
+// call g (see act_bwd_sn_kernel).  `group` counts elements (scalar kernel) or float4s (vector kernel) per call.
+struct ActFold {
+  float* acc;
+  const float* scale;      // per-call 1/sigma, or null (scale 1)
+  const float* bias;       // null: no bias
+  double* zw;              // null: no <G, W~> accumulation
+  size_t group;
+  int first;               // 1: acc is written, 0: acc is read, added to and written
+};
+
+template <bool FOLD>
 __global__ void act_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ y, float* __restrict__ dz,
-                               float* __restrict__ dbias, size_t total, int N, int act, float slope) {
+                               float* __restrict__ dbias, size_t total, int N, int act, float slope, ActFold f) {
   mtd_pdl_prologue();
   extern __shared__ float colsum[];   // N floats when dbias != null
   if (dbias) {
@@ -1191,9 +1204,22 @@ __global__ void act_bwd_kernel(const float* __restrict__ dy, const float* __rest
   size_t stride = (size_t)gridDim.x * blockDim.x;
   const bool fixed = dbias && (stride % (size_t)N == 0);   // channel of this thread never changes
   float priv = 0.f;
+  double part[4] = {0.0, 0.0, 0.0, 0.0};                     // FOLD: up to 4 batched calls
   for (; i < total; i += stride) {
     float g = dy[i];
-    if (act != MTD_ACT_NONE) g *= mtd_act_grad(__ldg(y + i), act, slope);
+    if constexpr (FOLD) {
+      const float t = (act != MTD_ACT_NONE || f.zw) ? __ldg(y + i) : 0.f;
+      if (act != MTD_ACT_NONE) g *= mtd_act_grad(t, act, slope);
+      const int gi = (i >= f.group) + (i >= 2 * f.group) + (i >= 3 * f.group);
+      const float a = f.scale ? __ldg(f.scale + gi) : 1.f;
+      f.acc[i] = f.first ? g * a : f.acc[i] + g * a;
+      if (f.zw) {
+        const float yp = (act == MTD_ACT_LEAKY && !(t > 0.f)) ? t * (1.f / slope) : t;
+        part[gi] += (double)(g * (yp - (f.bias ? __ldg(f.bias + i % N) : 0.f)));
+      }
+    } else {
+      if (act != MTD_ACT_NONE) g *= mtd_act_grad(__ldg(y + i), act, slope);
+    }
     if (dz) dz[i] = g;
     if (dbias) {
       if (fixed) priv += g;
@@ -1209,6 +1235,16 @@ __global__ void act_bwd_kernel(const float* __restrict__ dy, const float* __rest
     for (int c = threadIdx.x; c < N; c += blockDim.x) {
       float v = colsum[c];
       if (v != 0.f) atomicAdd(dbias + c, v);
+    }
+  }
+  if constexpr (FOLD) {
+    if (f.zw) {
+      __shared__ double red[32];
+      const int ngroups = (int)((total + f.group - 1) / f.group);
+      for (int k = 0; k < ngroups && k < 4; ++k) {
+        const double r = block_sum(part[k], red);
+        if (threadIdx.x == 0 && r != 0.0) atomicAdd(f.zw + k, r);
+      }
     }
   }
 }
@@ -1263,11 +1299,15 @@ __global__ void __launch_bounds__(256) act_bwd_v4_kernel(const float4* __restric
 // <G_g, W_orig>/sigma_g = <G_g, W~_g>, the coefficient of the spectral-norm weight-gradient correction -- taken from data
 // this pass reads anyway instead of a separate pass over the packed gradient and the weight.  LeakyReLU is inverted
 // exactly (y_pre = y > 0 ? y : y / slope); not available for ReLU (y = 0 loses y_pre).  zw and dbias pre-zeroed.
+// FOLD (mtd_act_bwd_acc): dz is written unscaled, dz * dz_scale[g] goes to acc (written when acc_first, else added),
+// zw is optional and y may be null when act is none and zw is null.
+template <bool FOLD>
 __global__ void __launch_bounds__(256) act_bwd_sn_kernel(const float4* __restrict__ dy, const float4* __restrict__ y,
                                                          float4* __restrict__ dz, float* __restrict__ dbias,
                                                          const float4* __restrict__ bias, double* __restrict__ zw,
                                                          const float* __restrict__ dz_scale, size_t total4, size_t group4,
-                                                         int N4, int act, float slope) {
+                                                         int N4, int act, float slope, float4* __restrict__ acc,
+                                                         int acc_first) {
   mtd_pdl_prologue();
   extern __shared__ float colsum[];   // 4 * N4 floats when dbias != null
   __shared__ double red[32];
@@ -1284,7 +1324,7 @@ __global__ void __launch_bounds__(256) act_bwd_sn_kernel(const float4* __restric
   double part[4] = {0.0, 0.0, 0.0, 0.0};                     // up to 4 batched calls
   for (; i < total4; i += stride) {
     float4 g = __ldcs(dy + i);
-    const float4 t = __ldcs(y + i);
+    const float4 t = (FOLD && !y) ? make_float4(0.f, 0.f, 0.f, 0.f) : __ldcs(y + i);
     float4 yp = t;
     if (act == MTD_ACT_LEAKY) {
       g.x *= t.x > 0.f ? 1.f : slope; g.y *= t.y > 0.f ? 1.f : slope; g.z *= t.z > 0.f ? 1.f : slope; g.w *= t.w > 0.f ? 1.f : slope;
@@ -1292,15 +1332,27 @@ __global__ void __launch_bounds__(256) act_bwd_sn_kernel(const float4* __restric
       yp.z = t.z > 0.f ? t.z : t.z * inv_slope; yp.w = t.w > 0.f ? t.w : t.w * inv_slope;
     }
     const int gi = (i >= group4) + (i >= 2 * group4) + (i >= 3 * group4);      // groups <= 4
-    if (dz) {
+    if constexpr (FOLD) {
+      if (dz) dz[i] = g;
+      const float a = dz_scale ? __ldg(dz_scale + gi) : 1.f;
+      const float4 s = make_float4(g.x * a, g.y * a, g.z * a, g.w * a);
+      if (acc_first) {
+        acc[i] = s;
+      } else {
+        const float4 o = acc[i];
+        acc[i] = make_float4(o.x + s.x, o.y + s.y, o.z + s.z, o.w + s.w);
+      }
+    } else if (dz) {
       // dz_scale: write dz / sigma_g, so that dgrad needs no epilogue scale and ONE weight-gradient GEMM over the
       // whole batch yields sum_g G_g / sigma_g; the bias gradient and zw use the unscaled dz
       const float a = dz_scale ? __ldg(dz_scale + gi) : 1.f;
       dz[i] = make_float4(g.x * a, g.y * a, g.z * a, g.w * a);
     }
     priv.x += g.x; priv.y += g.y; priv.z += g.z; priv.w += g.w;
-    const float d = g.x * (yp.x - b4.x) + g.y * (yp.y - b4.y) + g.z * (yp.z - b4.z) + g.w * (yp.w - b4.w);
-    part[gi] += (double)d;
+    if (!FOLD || zw) {
+      const float d = g.x * (yp.x - b4.x) + g.y * (yp.y - b4.y) + g.z * (yp.z - b4.z) + g.w * (yp.w - b4.w);
+      part[gi] += (double)d;
+    }
   }
   if (dbias) {
     if (first < total4) {
@@ -1313,6 +1365,7 @@ __global__ void __launch_bounds__(256) act_bwd_sn_kernel(const float4* __restric
       if (v != 0.f) atomicAdd(dbias + c, v);
     }
   }
+  if (FOLD && !zw) return;
   const int ngroups = (int)((total4 + group4 - 1) / group4);
   for (int k = 0; k < ngroups && k < 4; ++k) {
     const double r = block_sum(part[k], red);
@@ -1575,6 +1628,35 @@ int mtd_conv_wgrad_finish(const float* gp, float* dw_ref, int transposed, int Co
   return MTD_OK;
 }
 
+// Grid of the scalar act_bwd kernel: with column sums, the grid stride is made a multiple of N when possible (N is a
+// power of two for every layer here), so that each thread's channel never changes.
+static int act_bwd_scalar_blocks(size_t total, int N, bool colsums) {
+  int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)mtd_sm_count() * 8);
+  if (colsums) {
+    size_t stride = (size_t)blocks * 256;
+    if (stride % N != 0 && (size_t)N <= stride) {
+      size_t s2 = stride / N * N;
+      if (s2 % 256 == 0 && s2 > 0) blocks = (int)(s2 / 256);
+    } else if ((size_t)N > stride) {
+      blocks = (N + 255) / 256;
+    }
+  }
+  return blocks;
+}
+
+// Grid of act_bwd_sn_kernel: its grid stride must be a multiple of N4 (fixed channels per thread); 0 if impossible.
+static int act_bwd_sn_blocks(size_t total4, int N4) {
+  int blocks = (int)std::min<size_t>((total4 + 255) / 256, (size_t)mtd_sm_count() * 4);
+  size_t stride = (size_t)blocks * 256;
+  if ((size_t)N4 > stride) blocks = (N4 + 255) / 256;
+  else if (stride % N4 != 0) {
+    size_t s2 = stride / N4 * N4;
+    while (s2 > 0 && s2 % 256 != 0) s2 -= N4;
+    blocks = (int)(s2 / 256);
+  }
+  return ((size_t)blocks * 256) % N4 == 0 ? blocks : 0;
+}
+
 // dz = dy * act'(y); dbias[N] (optional) = column sums of dz.  dz may be null (colsum only) and may
 // alias dy.  dbias_zeroed != 0: the caller guarantees dbias is already all zero (e.g. carved from one zeroed slab
 // per backward pass), which saves a memset node per layer.
@@ -1604,20 +1686,12 @@ int mtd_act_bwd(const float* dy, const float* y, float* dz, float* dbias, int db
     MTD_CHECK_LAUNCH();
     return MTD_OK;
   }
-  int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)mtd_sm_count() * 8);
   if (dbias) {
     MTD_REQUIRE(N <= 8192);
     if (!dbias_zeroed) MTD_CUDA(cudaMemsetAsync(dbias, 0, (size_t)N * sizeof(float), st));
-    // make the grid stride a multiple of N when possible (N is a power of two for every layer here)
-    size_t stride = (size_t)blocks * 256;
-    if (stride % N != 0 && (size_t)N <= stride) {
-      size_t s2 = stride / N * N;
-      if (s2 % 256 == 0 && s2 > 0) blocks = (int)(s2 / 256);
-    } else if ((size_t)N > stride) {
-      blocks = (N + 255) / 256;
-    }
   }
-  mtd_launch(act_bwd_kernel, blocks, 256, dbias ? N * sizeof(float) : 0, st, dy, y, dz, dbias, total, N, act, slope);
+  mtd_launch(act_bwd_kernel<false>, act_bwd_scalar_blocks(total, N, dbias != nullptr), 256, dbias ? N * sizeof(float) : 0, st,
+             dy, y, dz, dbias, total, N, act, slope, ActFold{});
   MTD_CHECK_LAUNCH();
   return MTD_OK;
 }
@@ -1633,19 +1707,39 @@ int mtd_act_bwd_sn(const float* dy, const float* y, float* dz, float* dbias, con
   cudaStream_t st = (cudaStream_t)stream;
   const size_t total4 = (size_t)M * N / 4;
   const int N4 = N / 4;
-  int blocks = (int)std::min<size_t>((total4 + 255) / 256, (size_t)mtd_sm_count() * 4);
-  size_t stride = (size_t)blocks * 256;
-  if ((size_t)N4 > stride) blocks = (N4 + 255) / 256;
-  else if (stride % N4 != 0) {
-    size_t s2 = stride / N4 * N4;
-    while (s2 > 0 && s2 % 256 != 0) s2 -= N4;
-    MTD_REQUIRE(s2 > 0);
-    blocks = (int)(s2 / 256);
-  }
-  MTD_REQUIRE(((size_t)blocks * 256) % N4 == 0);
-  mtd_launch(act_bwd_sn_kernel, blocks, 256, dbias ? N * sizeof(float) : 0, st, reinterpret_cast<const float4*>(dy),
+  const int blocks = act_bwd_sn_blocks(total4, N4);
+  MTD_REQUIRE(blocks > 0);
+  mtd_launch(act_bwd_sn_kernel<false>, blocks, 256, dbias ? N * sizeof(float) : 0, st, reinterpret_cast<const float4*>(dy),
              reinterpret_cast<const float4*>(y), reinterpret_cast<float4*>(dz), dbias, reinterpret_cast<const float4*>(bias), zw,
-             dz_scale, total4, total4 / groups, N4, act, slope);
+             dz_scale, total4, total4 / groups, N4, act, slope, static_cast<float4*>(nullptr), 0);
+  MTD_CHECK_LAUNCH();
+  return MTD_OK;
+}
+
+// One backward pass's activation backward that also folds dz into accumulators spanning several passes (see the
+// header).  Same dz as mtd_act_bwd; N % 4 == 0 with 16-byte aligned operands takes the float4 kernel, anything else
+// the scalar one.
+int mtd_act_bwd_acc(const float* dy, const float* y, float* dz, float* acc, int acc_first, float* dbias, const float* bias,
+                    double* zw, const float* inv_sigma, int groups, long long M, int N, int act, float slope, void* stream) {
+  MTD_REQUIRE(dy && acc && M > 0 && N > 0 && N <= 8192 && groups >= 1 && groups <= 4 && M % groups == 0);
+  MTD_REQUIRE(y || (act == MTD_ACT_NONE && !zw));
+  MTD_REQUIRE(!zw || act == MTD_ACT_NONE || act == MTD_ACT_LEAKY);
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t total = (size_t)M * N;
+  if (N % 4 == 0 && mtd_aligned16(dy) && mtd_aligned16(acc) && (!y || mtd_aligned16(y)) && (!dz || mtd_aligned16(dz)) &&
+      (!bias || mtd_aligned16(bias))) {
+    const size_t total4 = total / 4;
+    const int N4 = N / 4;
+    const int blocks = act_bwd_sn_blocks(total4, N4);
+    MTD_REQUIRE(blocks > 0);
+    mtd_launch(act_bwd_sn_kernel<true>, blocks, 256, dbias ? N * sizeof(float) : 0, st, reinterpret_cast<const float4*>(dy),
+               reinterpret_cast<const float4*>(y), reinterpret_cast<float4*>(dz), dbias, reinterpret_cast<const float4*>(bias),
+               zw, inv_sigma, total4, total4 / groups, N4, act, slope, reinterpret_cast<float4*>(acc), acc_first);
+  } else {
+    const ActFold f{acc, inv_sigma, bias, zw, total / groups, acc_first};
+    mtd_launch(act_bwd_kernel<true>, act_bwd_scalar_blocks(total, N, dbias != nullptr), 256, dbias ? N * sizeof(float) : 0,
+               st, dy, y, dz, dbias, total, N, act, slope, f);
+  }
   MTD_CHECK_LAUNCH();
   return MTD_OK;
 }

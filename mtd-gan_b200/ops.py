@@ -287,6 +287,146 @@ def _flush_finish(groups):
     call("mtd_wgrad_finish_batched", ptr(seg), len(rows), ptr(ent[0]), ent[1], ptr(ent[2]), ent[3], ptr(dots), stream())
 
 
+# Task-gradient fold.  PCGrad needs, besides the per-task gradients of the shared parameters, the gradient of the SUM of
+# the task losses for the task-specific parameters.  Each task-specific layer lies on the path from some task loss to
+# the shared encoder, so the per-task backward passes already compute its dz (the gradient at its pre-activation) for
+# their task; its weight gradient (x (x) dz), bias gradient (sum dz) and spectral-norm correction (linear in G) are
+# linear in dz, and the activation masks are the same in every pass.  Inside `fold_task_grads(params)` a layer whose
+# weight is in `params` folds each pass's dz into one accumulator per forward instance (mtd_act_bwd_acc, in place of
+# its plain activation backward) and issues nothing for its weight; one weight-gradient GEMM per instance and one
+# batched finishing pass then give the same gradients as a separate backward pass of the summed loss, without it.
+_fold = None                  # the active fold_task_grads, or None
+
+
+class _FoldRec:
+    """One forward instance (autograd node) of a folded layer."""
+
+    def __init__(self, node, weight, x1, x2, dz_like, bias_grad, inv_sigma, u, v, zw, cfg, shapes):
+        self.node = node                    # keeps id(node), the record's key, from being reused
+        self.weight, self.x1, self.x2 = weight, x1, x2
+        self.acc = _empty(dz_like.shape, dz_like)
+        self.bias_grad, self.inv_sigma, self.u, self.v, self.zw = bias_grad, inv_sigma, u, v, zw
+        self.cfg, self.shapes = cfg, shapes
+        self.gp = None                      # packed weight gradient, once its GEMM is issued
+
+
+class fold_task_grads:
+    """Folds the task-specific gradients of several backward passes over one graph (see above).  Set `last_pass`
+    before the final pass: each instance's weight-gradient GEMM is then issued as soon as that pass has folded it, and
+    runs on the side stream alongside the rest of the pass.  After the context exits, `grads` holds the gradient of
+    every parameter in `params`, in order."""
+
+    def __init__(self, params):
+        self.params = list(params)
+        self.ptrs = {p.data_ptr() for p in self.params}
+        self.records = {}                   # id(autograd node) -> _FoldRec
+        self.bias_grads = {}                # bias data_ptr -> accumulated gradient (zeroed slab slice)
+        self.last_pass = False
+        self.grads = None
+        self._fslab = self._dslab = None
+
+    def __enter__(self):
+        global _fold
+        self.prev, _fold = _fold, self
+        return self
+
+    def __exit__(self, *exc):
+        global _fold
+        _fold = self.prev
+        if exc[0] is None:
+            self.grads = self._finish()
+        self.records = {}
+        return False
+
+    def wants(self, weight) -> bool:
+        return weight.data_ptr() in self.ptrs
+
+    def _zeros(self, n, dtype, like):
+        """n zeroed entries carved from one slab per fold (one memset instead of one per accumulator)."""
+        f = dtype == torch.float32
+        slab = self._fslab if f else self._dslab
+        if slab is None:
+            slab = [torch.zeros(1 << 16 if f else 1024, dtype=dtype, device=like.device), 0]
+            if f:
+                self._fslab = slab
+            else:
+                self._dslab = slab
+        step = (n + 63) // 64 * 64                     # 256-byte aligned slices
+        if slab[1] + step > slab[0].numel():
+            return torch.zeros(n, dtype=dtype, device=like.device)
+        t = slab[0][slab[1]:slab[1] + n]
+        slab[1] += step
+        return t
+
+    def act_bwd(self, node, g1, pre_out, weight, bias, want_bias, inv_sigma, u, v, x1, x2, cfg: "ConvCfg", shapes, has_add):
+        """Activation backward of a folded layer: returns this pass's (unscaled) dz and folds it into the instance's
+        accumulators."""
+        sn = inv_sigma is not None
+        G = inv_sigma.numel() if sn else 1
+        rec = self.records.get(id(node))
+        first = rec is None
+        if first:
+            if sn and (has_add or cfg.post_act != ACT_NONE or cfg.pre_act not in (ACT_NONE, ACT_LEAKY) or G > 4):
+                raise _ext.MtdError(f"task-gradient fold: no kernel for a spectrally-normalised layer with {cfg}")
+            bias_grad = None
+            if want_bias:
+                bias_grad = self.bias_grads.get(bias.data_ptr())
+                if bias_grad is None:
+                    bias_grad = self.bias_grads[bias.data_ptr()] = self._zeros(cfg.cout, torch.float32, g1)
+            zw = self._zeros(G, torch.float64, g1) if sn else None
+            rec = self.records[id(node)] = _FoldRec(node, weight, x1, x2, g1, bias_grad, inv_sigma, u, v, zw, cfg, shapes)
+        act = cfg.pre_act
+        dz = _empty(g1.shape, g1) if act != ACT_NONE else g1
+        y_in = pre_out if (act != ACT_NONE or sn) else None
+        call("mtd_act_bwd_acc", fptr(g1), fptr(y_in), fptr(dz) if act != ACT_NONE else None, fptr(rec.acc), 1 if first else 0,
+             fptr(rec.bias_grad), fptr(bias) if sn else None, ptr(rec.zw), fptr(inv_sigma), G, g1.numel() // cfg.cout,
+             cfg.cout, act, cfg.slope, stream())
+        if self.last_pass:
+            self._issue_wgrad(rec)
+        return dz
+
+    def _issue_wgrad(self, rec):
+        """One weight-gradient GEMM over the whole accumulated batch (pre-scaled by 1/sigma of each call)."""
+        if rec.gp is not None:
+            return
+        B, H, W, C1, C2 = rec.shapes
+        rec.gp = gp = _empty((rec.weight.numel(),), rec.acc)
+        launch = lambda: _conv_wgrad_launch(rec.x1, rec.x2, rec.acc, gp, B, H, W, C1, C2, rec.cfg)
+        if _WGRAD_SIDE and _finish_queue is not None and not torch.is_anomaly_enabled():
+            _on_side_stream(launch, rec.x1, rec.x2, rec.acc, gp)       # joined when the deferred-finishing pass exits
+        else:
+            launch()
+
+    def _finish(self):
+        groups = {}
+        for rec in self.records.values():
+            self._issue_wgrad(rec)
+            w = rec.weight.detach()
+            if rec.inv_sigma is not None:
+                u, v, G = rec.u, rec.v, rec.inv_sigma.numel()
+                insts = [(rec.gp if g == 0 else None, w, u[g] if u.dim() == 2 else u, v[g] if v.dim() == 2 else v,
+                          rec.inv_sigma[g:g + 1], rec.cfg, rec.zw.data_ptr() + 8 * g, 2 if g == 0 else 4) for g in range(G)]
+            else:
+                insts = [(rec.gp, w, None, None, None, rec.cfg, 0, 0)]
+            grp = groups.get(w.data_ptr())
+            if grp is None:
+                groups[w.data_ptr()] = (torch.empty_like(w), insts)
+            else:
+                grp[1].extend(insts)            # instances of one weight are summed by the batched finishing pass
+        _join_side_stream()
+        if groups:
+            _flush_finish(groups)
+        out = []
+        for p in self.params:
+            g = groups.get(p.data_ptr())
+            g = g[0] if g is not None else self.bias_grads.get(p.data_ptr())
+            if g is None:
+                raise _ext.MtdError(f"task-gradient fold: parameter of shape {tuple(p.shape)} was reached by no backward "
+                                    "pass (it is not used in the graph of the losses)")
+            out.append(g)
+        return out
+
+
 @dataclass(frozen=True)
 class ConvCfg:
     cin: int                 # total input channels (C1 + C2)
@@ -500,6 +640,11 @@ class ConvFn(Function):
             g1 = _empty(dy.shape, dy)
             call("mtd_act_bwd", fptr(dy), fptr(y), fptr(g1), None, 0, M, cfg.cout, cfg.post_act, cfg.slope, st)
         d_add = g1 if ctx.has_add else None
+        folded = _fold is not None and need[2] and _fold.wants(weight)
+        if folded:         # weight and bias gradients are folded across the passes (fold_task_grads), none is issued here
+            dz = _fold.act_bwd(ctx, g1, aux if aux is not None else y, weight, bias, need[3], inv_sigma, u, v, x1, x2, cfg,
+                               ctx.shapes, ctx.has_add)
+            need[2] = need[3] = False
         dbias, dbz = _dbias_alloc(cfg.cout, dy) if need[3] else (None, 0)
         want_w = need[2] and _wgrad_wanted(weight)
         G = 1 if inv_sigma is None else inv_sigma.numel()
@@ -512,7 +657,9 @@ class ConvFn(Function):
         if (want_w and inv_sigma is not None and deferred and cfg.post_act == ACT_NONE and not ctx.has_add
                 and cfg.pre_act in (ACT_NONE, ACT_LEAKY) and cfg.cout % 4 == 0 and G <= 4):
             zw = _zw_alloc(G, dy)
-        if zw is not None:
+        if folded:
+            pass
+        elif zw is not None:
             if dbias is not None and not dbz:
                 dbias.zero_()
             # dz is written pre-scaled by 1/sigma of its call: dgrad then needs no scale, and ONE weight-gradient GEMM over

@@ -1,8 +1,9 @@
 """PCGrad weight method on the B200 path — the surface train.py / engine.py use
 (`WeightMethods('pcgrad', n_tasks=3, device=...)`, module/weight_methods.py:409-468, 727-761).
 
-The per-task backward passes still go through torch.autograd.grad (three over the shared parameters,
-one over the task-specific ones, like the reference :432-433, :443), but the projection itself runs in
+The per-task backward passes still go through torch.autograd.grad (one per task over the shared parameters, like
+the reference :432-433).  The reference's fourth pass over the task-specific parameters (:443) is not run: those
+gradients are folded from the per-task passes (ops.fold_task_grads).  The projection runs in
 Gram space on the device: one pass for the T(T+1)/2 dots, a one-thread solve that replays the
 reference's shuffle/dot/project loop, one combine pass.  The host never reads a dot product back, so the
 `if g_i_g_j < 0` host sync of the reference (:455) is gone.  Python's global `random` is consumed exactly
@@ -18,7 +19,7 @@ import torch
 from . import _ext
 from . import distributed as mdist
 from ._ext import call, fptr, ptr, stream
-from .ops import deferred_wgrad_finish, wgrad_only_for
+from .ops import deferred_wgrad_finish, fold_task_grads, wgrad_only_for
 
 
 def draw_visit_orders(n_tasks: int, rng=None) -> List[List[int]]:
@@ -156,7 +157,13 @@ class WeightMethod:
 
 
 class PCGrad(WeightMethod):
-    """module/weight_methods.py:409-468."""
+    """module/weight_methods.py:409-468.
+
+    One backward pass per task (torch.autograd.grad over the shared parameters) gives the per-task shared gradients,
+    projected in Gram space on the device.  The same passes fold the gradient of losses.sum() for the task-specific
+    parameters (ops.fold_task_grads: their weight gradient is linear in each layer's dz, which every pass computes
+    anyway), so the reference's fourth backward pass (:443) is not run; its result is the same up to fp32 summation
+    order.  A task-specific parameter that no task loss reaches raises, like the reference's autograd.grad."""
 
     def __init__(self, n_tasks: int, device: torch.device, reduction="sum"):
         super().__init__(n_tasks, device=device)
@@ -176,39 +183,34 @@ class PCGrad(WeightMethod):
             task_specific_parameters = list(task_specific_parameters)
         if mdist.active():
             return self._set_pc_grads_distributed(losses, shared_parameters, task_specific_parameters)
-        # shared part (:431-439): one backward pass per task, weight-gradient GEMMs only for the shared set
+        # shared part (:431-439): one backward pass per task, weight-gradient GEMMs only for the shared set; the task
+        # specific part (:442-447, the gradient of losses.sum()) is folded from the same passes
         shared_grads = []
-        with wgrad_only_for(shared_parameters):
-            for l in losses:
+        with wgrad_only_for(shared_parameters), fold_task_grads(task_specific_parameters or []) as fold:
+            for k, l in enumerate(losses):
+                fold.last_pass = k + 1 == len(losses)
                 with deferred_wgrad_finish():        # one batched finishing pass per task backward
-                    shared_grads.append(torch.autograd.grad(l, shared_parameters, retain_graph=True))
+                    shared_grads.append(torch.autograd.grad(l, shared_parameters, retain_graph=not fold.last_pass))
         merged = self._project_conflicting(shared_grads)
         for p, g in zip(shared_parameters, merged):
             p.grad = g
-        # task specific part (:442-447)
         if task_specific_parameters is not None:
-            with wgrad_only_for(task_specific_parameters), deferred_wgrad_finish():
-                ts_grads = torch.autograd.grad(losses.sum(), task_specific_parameters)
-            for p, g in zip(task_specific_parameters, ts_grads):
+            for p, g in zip(task_specific_parameters, fold.grads):
                 p.grad = g
 
     def _set_pc_grads_distributed(self, losses, shared_parameters, task_specific_parameters):
         """Same gradients as the single-process path on the concatenated batch (SURVEY §8e), with the collectives
-        overlapped: the four backward passes are independent `autograd.grad` calls, so the task-specific one runs FIRST
-        and its all-reduce, like the reduce-scatter of each task's shared gradients, proceeds on the communication
-        stream while the next backward pass computes (distributed.py)."""
-        ts_pending = None
-        if task_specific_parameters is not None:
-            with wgrad_only_for(task_specific_parameters), deferred_wgrad_finish():
-                ts_grads = torch.autograd.grad(losses.sum(), task_specific_parameters, retain_graph=True)
-            ts_pending = mdist.allreduce_mean_list_async(ts_grads)
+        overlapped: the reduce-scatter of each task's shared gradients proceeds on the communication stream while the
+        next backward pass computes (distributed.py).  The all-reduce of the folded task-specific gradients follows the
+        last pass and overlaps the sharded projection."""
         pipe = mdist.ShardedPCGrad()
-        n = len(losses)
-        with wgrad_only_for(shared_parameters):
+        with wgrad_only_for(shared_parameters), fold_task_grads(task_specific_parameters or []) as fold:
             for k, l in enumerate(losses):
+                fold.last_pass = k + 1 == len(losses)
                 with deferred_wgrad_finish():
-                    g = torch.autograd.grad(l, shared_parameters, retain_graph=(k + 1 < n))
+                    g = torch.autograd.grad(l, shared_parameters, retain_graph=not fold.last_pass)
                 pipe.submit(g)
+        ts_pending = mdist.allreduce_mean_list_async(fold.grads) if task_specific_parameters is not None else None
         orders = self.refresh_orders(shared_parameters[0].device)
         merged = pipe.finish(orders, self.reduction == "mean", _cuda_gram, _cuda_solve_combine)
         for p, g in zip(shared_parameters, merged):
