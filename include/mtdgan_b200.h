@@ -163,8 +163,10 @@ int mtd_split_tf32(float* hi, float* lo, long long n, void* stream);
 /* ---- Res-FFT-Conv frequency branch (fft_block.cu) ------------------------------------------------
  * Replaces torch.fft.rfft2 / cat / fft_conv 1x1 + ReLU / chunk / complex / torch.fft.irfft2 at
  * arch/Ours/networks.py:24-29 and their autograd backward.  Half spectrum layout:
- * spec[B][W/2+1][H][C] complex64 (interleaved).  H, W powers of two; C == 32 for the mix.          */
-/* 1 when the frequency branch supports the geometry: C == 32 and H, W in {64, 128, 256, 512} (four-step FFTs 8x8 ... 16x32) */
+ * spec[B][W/2+1][H][C] complex64 (interleaved); C == 32 for the mix.                              */
+/* 1 when the frequency branch supports the geometry: C == 32 and 1 <= H, W <= 512.  Lengths 64, 128, 256, 512 run four-step
+ * FFTs (8x8 ... 16x32); every other length a Bluestein transform on a power-of-two length up to 1024.  The backward
+ * (mtd_fft_cols_mix_bwd) takes H in {64, 128, 256} and W in {64, 128, 256, 512} only. */
 int mtd_fft_supported(int H, int W, int C);
 long long mtd_fft_spec_elems(int B, int H, int W, int C);          /* floats in a spectrum buffer      */
 long long mtd_fft_bwd_part_elems(int B, int W);                    /* floats in the bwd partial buffer */

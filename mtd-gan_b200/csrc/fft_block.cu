@@ -20,8 +20,13 @@
 //   * columns: lane = channel, so every shared-memory access is a 256-byte row (conflict-free); the spectrum stays
 //     in [k1][k2] order between the forward and the inverse transform -- the channel mix is frequency-local, so no
 //     reordering pass exists.
-// Supported lengths: 64, 128, 256, 512 (8x8, 8x16, 16x16, 16x32).
+// Lengths 64, 128, 256, 512 run these kernels (8x8, 8x16, 16x16, 16x32).  Every other length 1 <= N <= 512 runs the
+// Bluestein kernels further down (forward only): P1 / P3 as one chirp-z transform per image row, P2 split into a
+// column transform, a flat channel-mix pass and an inverse column transform.
 #include <algorithm>
+#include <cmath>
+#include <mutex>
+#include <vector>
 #include "common.cuh"
 #include "fft_core.cuh"
 #include "mtdgan_b200.h"
@@ -562,6 +567,276 @@ __global__ void __launch_bounds__(256) fft_wgrad_reduce_kernel(const float* __re
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Bluestein (chirp-z) transforms for every other length N <= 512:
+//   X[k] = c[k] sum_n (x[n] c[n]) conj(c[k - n]),   c[n] = exp(-i pi n^2 / N)
+// The convolution runs circularly at M = max(64, pow2 >= 2N - 1) <= 1024 on the four-step transforms above:
+//   step A   thread (n2, l): x[n] c[n] at n = N2*n1 + n2 (0 for n >= N), N1-point FFT, twiddle -> S[k1][n2]
+//   step BA  thread (k1, l): N2-point FFT, * Bh[k1 + N1*k2], N2-point inverse FFT, conj twiddle -> S[k1][n2] in place
+//            (the pointwise product is frequency-local, so the forward and the inverse transform meet in registers)
+//   step B'  thread (n2, l): N1-point inverse FFT, * c[n] -> store(n, l, .) for n < N, after a barrier (S is free)
+// Bh = FFT_M(conj(c) wrapped circularly) / M.  INV (the unnormalised inverse DFT) uses conj(c) and conj(Bh): the wrapped
+// chirp is symmetric, so FFT_M of its conjugate is conj(Bh).
+// kNL = 16 interleaved complex sequences per CTA: the 16 channel pairs of one image row, or 16 channels of one (b, kw)
+// column slice.  S[M][16] is 128 KB at M = 1024.
+// ------------------------------------------------------------------------------------------------
+constexpr int kNL = 16;
+
+template <int N1, int N2>
+struct BlueCfg {
+  static constexpr int M = N1 * N2;
+  static constexpr int THREADS = (N1 > N2 ? N1 : N2) * kNL;          // at most one item per thread in every step
+  static constexpr size_t smem = (size_t)M * kNL * 8 + (size_t)M * 8;   // S | tw
+};
+
+template <int N1, int N2, bool INV, class Load, class Store>
+__device__ __forceinline__ void bluestein(float2* S, float2* tw, const float2* __restrict__ chirp, const float2* __restrict__ bh,
+                                          int N, Load load, Store store) {
+  constexpr int M = N1 * N2;
+  const int l = threadIdx.x & (kNL - 1), t = threadIdx.x / kNL;
+  fill_twiddles(tw, M);
+  __syncthreads();
+  if (t < N2) {                                                        // step A
+    const int n2 = t;
+    float2 v[N1];
+#pragma unroll
+    for (int n1 = 0; n1 < N1; ++n1) {
+      const int n = N2 * n1 + n2;
+      v[n1] = make_float2(0.f, 0.f);
+      if (n < N) {
+        const float2 x = load(n, l), c = __ldg(chirp + n);
+        v[n1] = INV ? cmulc(x, c) : cmul(x, c);
+      }
+    }
+    fft_reg<N1, false>(v);
+#pragma unroll
+    for (int i = 0; i < N1; ++i) {
+      const int k1 = brev_c(i, N1);
+      S[(k1 * N2 + n2) * kNL + l] = k1 == 0 ? v[i] : cmul(v[i], tw[(n2 * k1) & (M - 1)]);
+    }
+  }
+  __syncthreads();
+  if (t < N1) {                                                        // step BA
+    const int k1 = t;
+    float2 v[N2], z[N2];
+#pragma unroll
+    for (int n2 = 0; n2 < N2; ++n2) v[n2] = S[(k1 * N2 + n2) * kNL + l];
+    fft_reg<N2, false>(v);                                             // v[j] = Y[k1 + N1 * brev(j)]
+#pragma unroll
+    for (int j = 0; j < N2; ++j) {
+      const int k2 = brev_c(j, N2);
+      const float2 b = __ldg(bh + k1 + N1 * k2);
+      z[k2] = INV ? cmulc(v[j], b) : cmul(v[j], b);
+    }
+    fft_reg<N2, true>(z);                                              // z[j] = y[k1][n2 = brev(j)]
+#pragma unroll
+    for (int j = 0; j < N2; ++j) {
+      const int n2 = brev_c(j, N2);
+      S[(k1 * N2 + n2) * kNL + l] = k1 == 0 ? z[j] : cmulc(z[j], tw[(n2 * k1) & (M - 1)]);
+    }
+  }
+  __syncthreads();
+  float2 v[N1];                                                        // step B'
+  const int n2 = t;
+  if (t < N2) {
+#pragma unroll
+    for (int k1 = 0; k1 < N1; ++k1) v[k1] = S[(k1 * N2 + n2) * kNL + l];
+    fft_reg<N1, true>(v);                                              // v[i] = y[n2 + N2 * brev(i)]
+  }
+  __syncthreads();
+  if (t < N2) {
+#pragma unroll
+    for (int i = 0; i < N1; ++i) {
+      const int n = n2 + N2 * brev_c(i, N1);
+      if (n < N) {
+        const float2 c = __ldg(chirp + n);
+        store(n, l, INV ? cmulc(v[i], c) : cmul(v[i], c));
+      }
+    }
+  }
+}
+
+// P1 at any W: one image row per CTA.  grid = B*H
+template <int N1, int N2>
+__global__ void __launch_bounds__(BlueCfg<N1, N2>::THREADS) fft_rows_fwd_blue_kernel(const float* __restrict__ x, float2* __restrict__ spec,
+                                                                                    int H, int W, const float2* __restrict__ chirp,
+                                                                                    const float2* __restrict__ bh) {
+  mtd_pdl_prologue();
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float2* S = reinterpret_cast<float2*>(smem_raw);                     // [M][16]; Z[k][q] after the transform
+  float2* tw = S + (size_t)N1 * N2 * kNL;
+  const long long row = blockIdx.x;
+  const float2* src = reinterpret_cast<const float2*>(x + (size_t)row * W * kC);     // src[n * 16 + q] = (x_2q, x_2q+1)[n]
+  bluestein<N1, N2, false>(S, tw, chirp, bh, W, [&](int n, int q) { return __ldg(src + (size_t)n * kQ + q); },
+                           [&](int k, int q, float2 z) { S[k * kNL + q] = z; });
+  __syncthreads();
+  // real-pair separation A_k = (Z_k + conj Z_{W-k}) / 2, B_k = -i (Z_k - conj Z_{W-k}) / 2 for k <= W/2
+  const int Wh = W / 2 + 1, b = (int)(row / H), h = (int)(row - (long long)b * H);
+  float2* dst0 = spec + ((size_t)b * Wh * H + h) * kC;
+  const float sc = rsqrtf((float)W) * 0.5f;
+  for (int i = threadIdx.x; i < Wh * kQ; i += blockDim.x) {
+    const int k = i / kQ, q = i % kQ;
+    const float2 zk = S[k * kNL + q];
+    float2 zm = S[(k == 0 ? 0 : W - k) * kNL + q];
+    zm.y = -zm.y;
+    const float4 o = make_float4((zk.x + zm.x) * sc, (zk.y + zm.y) * sc, (zk.y - zm.y) * sc, -(zk.x - zm.x) * sc);
+    *reinterpret_cast<float4*>(dst0 + (size_t)k * H * kC + 2 * q) = o;
+  }
+}
+
+// P3 at any W: one image row per CTA, fused residual adds.  grid = B*H.  The imaginary parts of kw = 0, and of kw = W/2
+// when W is even, are dropped (SURVEY A1); an odd W has no Nyquist column.
+template <int N1, int N2>
+__global__ void __launch_bounds__(BlueCfg<N1, N2>::THREADS) fft_rows_inv_blue_kernel(const float2* __restrict__ spec,
+                                                                                    const float* __restrict__ add1,
+                                                                                    const float* __restrict__ add2,
+                                                                                    float* __restrict__ out, int H, int W,
+                                                                                    const float2* __restrict__ chirp,
+                                                                                    const float2* __restrict__ bh) {
+  mtd_pdl_prologue();
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float2* S = reinterpret_cast<float2*>(smem_raw);
+  float2* tw = S + (size_t)N1 * N2 * kNL;
+  const long long row = blockIdx.x;
+  const int Wh = W / 2 + 1, b = (int)(row / H), h = (int)(row - (long long)b * H);
+  const float2* src0 = spec + ((size_t)b * Wh * H + h) * kC;
+  const float sc = rsqrtf((float)W);
+  const size_t base = (size_t)row * W * kC;
+  bluestein<N1, N2, true>(
+      S, tw, chirp, bh, W,
+      [&](int n, int q) {                                              // Z[n] = A_n + i B_n;  Z[W-n] = conj(A_n) + i conj(B_n)
+        const bool up = n >= Wh;
+        const float4 v = __ldg(reinterpret_cast<const float4*>(src0 + (size_t)(up ? W - n : n) * H * kC + 2 * q));
+        if (n == 0 || 2 * n == W) return make_float2(v.x, v.z);
+        return up ? make_float2(v.x + v.w, v.z - v.y) : make_float2(v.x - v.w, v.y + v.z);
+      },
+      [&](int n, int q, float2 z) {
+        const size_t o = base + (size_t)n * kC + 2 * q;
+        float2 val = make_float2(z.x * sc, z.y * sc);
+        if (add1) { const float2 a = __ldg(reinterpret_cast<const float2*>(add1 + o)); val.x += a.x; val.y += a.y; }
+        if (add2) { const float2 a = __ldg(reinterpret_cast<const float2*>(add2 + o)); val.x += a.x; val.y += a.y; }
+        *reinterpret_cast<float2*>(out + o) = val;
+      });
+}
+
+// P2 at any H, column transform of 16 channels of one (b, kw) slice: out = scale * DFT_H(in) (INV: inverse DFT).
+// grid = 2 * B*Wh.  May run in place (in == out): a CTA reads its columns before it writes them.
+template <int N1, int N2, bool INV>
+__global__ void __launch_bounds__(BlueCfg<N1, N2>::THREADS) fft_cols_blue_kernel(const float2* in, float2* out, int H, float scale,
+                                                                                const float2* __restrict__ chirp,
+                                                                                const float2* __restrict__ bh) {
+  mtd_pdl_prologue();
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float2* S = reinterpret_cast<float2*>(smem_raw);
+  float2* tw = S + (size_t)N1 * N2 * kNL;
+  const size_t off = (size_t)(blockIdx.x >> 1) * H * kC + (blockIdx.x & 1) * kNL;
+  const float2* src = in + off;
+  float2* dst = out + off;
+  bluestein<N1, N2, INV>(S, tw, chirp, bh, H, [&](int n, int c) { return src[(size_t)n * kC + c]; },
+                         [&](int k, int c, float2 z) { dst[(size_t)k * kC + c] = make_float2(z.x * scale, z.y * scale); });
+}
+
+// P2 at any H, channel mix: every row of the spectrum is one frequency, mixed independently (in place):
+// row = relu(bias + row M), M = w / sqrt(H) in the interleaved index space.  128 rows per CTA.  grid = ceil(nrows / 128)
+constexpr int kMixRows = 128, kThreadsMix = 256;
+__global__ void __launch_bounds__(kThreadsMix) fft_mix_rows_kernel(float2* spec, const float* __restrict__ w, const float* __restrict__ bias,
+                                                                  long long nrows, float scale) {
+  mtd_pdl_prologue();
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float* Sf = reinterpret_cast<float*>(smem_raw);                      // [128][kMixLd]
+  float* Bhi = Sf + kMixRows * kMixLd;
+  float* Blo = Bhi + kC2 * kMixLd;
+  float* bs = Blo + kC2 * kMixLd;
+  mix_prepare(w, bias, scale, Bhi, Blo, bs);
+  const long long r0 = (long long)blockIdx.x * kMixRows;
+  float4* g = reinterpret_cast<float4*>(spec) + r0 * (kC2 / 4);
+  for (int i = threadIdx.x; i < kMixRows * (kC2 / 4); i += kThreadsMix) {
+    const int r = i / (kC2 / 4), c = i % (kC2 / 4);
+    *reinterpret_cast<float4*>(Sf + r * kMixLd + 4 * c) = r0 + r < nrows ? g[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  __syncthreads();
+  mix_mma<kMixRows, kThreadsMix, 0>(reinterpret_cast<float2*>(Sf), reinterpret_cast<float2*>(Sf), Bhi, Blo, bs);
+  __syncthreads();
+  for (int i = threadIdx.x; i < kMixRows * (kC2 / 4); i += kThreadsMix) {
+    const int r = i / (kC2 / 4), c = i % (kC2 / 4);
+    if (r0 + r < nrows) g[i] = *reinterpret_cast<const float4*>(Sf + r * kMixLd + 4 * c);
+  }
+}
+
+int blue_len(int n) {
+  int m = 64;
+  while (m < 2 * n - 1) m <<= 1;
+  return m;
+}
+
+// chirp c[n] (n < N) and Bh[k] (k < M) of a length, built once per (device, length) on the host in fp64 and kept on the
+// device for the life of the process (12 KB at most per length).  The phase pi n^2 / N is reduced as n^2 mod 2N in integer
+// arithmetic first: formed in fp32, it loses the phase at N ~ 500.
+struct BlueTables {
+  std::once_flag once;
+  int rc = MTD_OK;
+  float2* chirp = nullptr;
+  float2* bh = nullptr;
+};
+constexpr int kBlueMaxDev = 16;
+
+int blue_tables(int N, const float2** chirp, const float2** bh) {
+  static BlueTables tabs[kBlueMaxDev][513];
+  int dev = 0;
+  MTD_CUDA(cudaGetDevice(&dev));
+  if (dev >= kBlueMaxDev || N < 1 || N > 512) return MTD_EINVAL;
+  BlueTables& t = tabs[dev][N];
+  std::call_once(t.once, [&] {
+    const int M = blue_len(N);
+    std::vector<double> cr(M), ci(M), er(M), ei(M);            // cr + i ci: wrapped conj(c);  er + i ei = exp(-2 pi i j / M)
+    for (int j = 0; j < M; ++j) {
+      er[j] = std::cos(2.0 * M_PI * j / M);
+      ei[j] = -std::sin(2.0 * M_PI * j / M);
+    }
+    std::vector<float2> hc(N), hb(M);
+    for (int n = 0; n < N; ++n) {
+      const double a = M_PI * (double)(((long long)n * n) % (2LL * N)) / N;
+      hc[n] = make_float2((float)std::cos(a), (float)-std::sin(a));
+      cr[n] = std::cos(a);
+      ci[n] = std::sin(a);
+      if (n) { cr[M - n] = cr[n]; ci[M - n] = ci[n]; }
+    }
+    for (int k = 0; k < M; ++k) {
+      double sr = 0.0, si = 0.0;
+      for (int m = 0; m < M; ++m) {
+        if (m >= N && m <= M - N) continue;                    // the zero padding
+        const int j = (int)(((long long)m * k) % M);
+        sr += cr[m] * er[j] - ci[m] * ei[j];
+        si += cr[m] * ei[j] + ci[m] * er[j];
+      }
+      hb[k] = make_float2((float)(sr / M), (float)(si / M));
+    }
+    float2 *dc = nullptr, *db = nullptr;
+    cudaError_t e = cudaMalloc(&dc, sizeof(float2) * N);
+    if (e == cudaSuccess) e = cudaMalloc(&db, sizeof(float2) * M);
+    if (e == cudaSuccess) e = cudaMemcpy(dc, hc.data(), sizeof(float2) * N, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(db, hb.data(), sizeof(float2) * M, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();        // the copies complete before any stream can read them
+    t.rc = (int)e;
+    t.chirp = dc;
+    t.bh = db;
+  });
+  *chirp = t.chirp;
+  *bh = t.bh;
+  return t.rc;
+}
+
+// dispatch on the Bluestein convolution length M = N1 x N2
+#define MTD_BLUE_DISPATCH(M, CALL)      \
+  switch (M) {                          \
+    case 64: { CALL(8, 8); break; }     \
+    case 128: { CALL(8, 16); break; }   \
+    case 256: { CALL(16, 16); break; }  \
+    case 512: { CALL(16, 32); break; }  \
+    case 1024: { CALL(32, 32); break; } \
+    default: return MTD_EINVAL;         \
+  }
+
 template <typename K>
 int set_smem(K kernel, size_t bytes) {
   if (bytes > 227 * 1024) return MTD_EINVAL;
@@ -584,6 +859,24 @@ bool fft_len_ok(int n) { return n == 64 || n == 128 || n == 256 || n == 512; }
     default: return MTD_EINVAL;       \
   }
 
+// P2 column transforms at any H: out = scale * DFT_H(in) (INV: the inverse DFT) over every (b, kw) slice
+template <bool INV>
+int launch_cols_blue(const float2* in, float2* out, int nslices, int H, float scale, const float2* chirp, const float2* bh,
+                     cudaStream_t st) {
+#define CALL(N1_, N2_)                                                                                              \
+  {                                                                                                                 \
+    using Cfg = BlueCfg<N1_, N2_>;                                                                                  \
+    int rc = set_smem(fft_cols_blue_kernel<N1_, N2_, INV>, Cfg::smem);                                              \
+    if (rc) return rc;                                                                                              \
+    mtd_launch(fft_cols_blue_kernel<N1_, N2_, INV>, 2 * nslices, Cfg::THREADS, Cfg::smem, st, in, out, H, scale,    \
+               chirp, bh);                                                                                          \
+  }
+  MTD_BLUE_DISPATCH(blue_len(H), CALL)
+#undef CALL
+  MTD_CHECK_LAUNCH();
+  return MTD_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -593,13 +886,30 @@ long long mtd_fft_spec_elems(int B, int H, int W, int C) { return (long long)B *
 // per-CTA dW / db partials followed by the four tf32 mix operands of the backward kernel
 long long mtd_fft_bwd_part_elems(int B, int W) { return (long long)B * (W / 2 + 1) * (kC2 * kC2 + kC2) + 4LL * kC2 * kMixLd; }
 
-/* 1 when (H, W, C) is a geometry the frequency branch supports: C == 32, H and W in {64, 128, 256, 512}. */
-int mtd_fft_supported(int H, int W, int C) { return (C == kC && fft_len_ok(H) && fft_len_ok(W)) ? 1 : 0; }
+/* 1 when (H, W, C) is a geometry the frequency branch supports: C == 32, 1 <= H, W <= 512. */
+int mtd_fft_supported(int H, int W, int C) { return (C == kC && H >= 1 && H <= 512 && W >= 1 && W <= 512) ? 1 : 0; }
 
 int mtd_fft_rows_fwd(const float* x, float* spec, int B, int H, int W, int C, void* stream) {
-  MTD_REQUIRE(x && spec && B > 0 && H > 0 && fft_len_ok(W) && C == kC);
+  MTD_REQUIRE(x && spec && B > 0 && H > 0 && W >= 1 && W <= 512 && C == kC);
   MTD_REQUIRE(mtd_aligned16(x) && mtd_aligned16(spec));
   const int nrows = B * H;
+  if (!fft_len_ok(W)) {
+    const float2 *chirp, *bh;
+    int rc = blue_tables(W, &chirp, &bh);
+    if (rc) return rc;
+#define CALL(N1_, N2_)                                                                                              \
+  {                                                                                                                 \
+    using Cfg = BlueCfg<N1_, N2_>;                                                                                  \
+    rc = set_smem(fft_rows_fwd_blue_kernel<N1_, N2_>, Cfg::smem);                                                   \
+    if (rc) return rc;                                                                                              \
+    mtd_launch(fft_rows_fwd_blue_kernel<N1_, N2_>, nrows, Cfg::THREADS, Cfg::smem, (cudaStream_t)stream, x,         \
+               reinterpret_cast<float2*>(spec), H, W, chirp, bh);                                                   \
+  }
+    MTD_BLUE_DISPATCH(blue_len(W), CALL)
+#undef CALL
+    MTD_CHECK_LAUNCH();
+    return MTD_OK;
+  }
 #define CALL(N1_, N2_)                                                                                              \
   {                                                                                                                 \
     using Cfg = RowsCfg<N1_, N2_>;                                                                                  \
@@ -616,9 +926,26 @@ int mtd_fft_rows_fwd(const float* x, float* spec, int B, int H, int W, int C, vo
 
 int mtd_fft_rows_inv(const float* spec, const float* add1, const float* add2, float* out, int B, int H, int W, int C,
                      void* stream) {
-  MTD_REQUIRE(spec && out && B > 0 && H > 0 && fft_len_ok(W) && C == kC);
+  MTD_REQUIRE(spec && out && B > 0 && H > 0 && W >= 1 && W <= 512 && C == kC);
   MTD_REQUIRE(mtd_aligned16(spec) && mtd_aligned16(out) && mtd_aligned16(add1) && mtd_aligned16(add2));
   const int nrows = B * H;
+  if (!fft_len_ok(W)) {
+    const float2 *chirp, *bh;
+    int rc = blue_tables(W, &chirp, &bh);
+    if (rc) return rc;
+#define CALL(N1_, N2_)                                                                                              \
+  {                                                                                                                 \
+    using Cfg = BlueCfg<N1_, N2_>;                                                                                  \
+    rc = set_smem(fft_rows_inv_blue_kernel<N1_, N2_>, Cfg::smem);                                                   \
+    if (rc) return rc;                                                                                              \
+    mtd_launch(fft_rows_inv_blue_kernel<N1_, N2_>, nrows, Cfg::THREADS, Cfg::smem, (cudaStream_t)stream,            \
+               reinterpret_cast<const float2*>(spec), add1, add2, out, H, W, chirp, bh);                           \
+  }
+    MTD_BLUE_DISPATCH(blue_len(W), CALL)
+#undef CALL
+    MTD_CHECK_LAUNCH();
+    return MTD_OK;
+  }
 #define CALL(N1_, N2_)                                                                                              \
   {                                                                                                                 \
     using Cfg = RowsCfg<N1_, N2_>;                                                                                  \
@@ -635,8 +962,30 @@ int mtd_fft_rows_inv(const float* spec, const float* add1, const float* add2, fl
 
 int mtd_fft_cols_mix(const float* spec_in, float* spec_out, const float* w, const float* bias, int B, int H, int W,
                      int C, void* stream) {
-  MTD_REQUIRE(spec_in && spec_out && w && bias && B > 0 && fft_len_ok(H) && W >= 2 && C == kC);
+  MTD_REQUIRE(spec_in && spec_out && w && bias && B > 0 && H >= 1 && H <= 512 && W >= 1 && W <= 512 && C == kC);
   MTD_REQUIRE(mtd_aligned16(spec_in) && mtd_aligned16(spec_out));
+  if (!fft_len_ok(H)) {
+    // column transform, flat channel mix, inverse column transform: a 32-channel M-row slice does not fit in shared
+    // memory at M = 1024, so the transforms run on 16-channel halves and the mix on the spectrum in global memory (L2)
+    const float2 *chirp, *bh;
+    int rc = blue_tables(H, &chirp, &bh);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nslices = B * (W / 2 + 1);
+    const float sH = 1.0f / sqrtf((float)H);
+    rc = launch_cols_blue<false>(reinterpret_cast<const float2*>(spec_in), reinterpret_cast<float2*>(spec_out), nslices, H,
+                                 1.0f, chirp, bh, st);
+    if (rc) return rc;
+    const size_t msmem = ((size_t)kMixRows * kMixLd + 2 * kC2 * kMixLd + kC2) * 4;
+    rc = set_smem(fft_mix_rows_kernel, msmem);
+    if (rc) return rc;
+    const long long nrows = (long long)nslices * H;
+    mtd_launch(fft_mix_rows_kernel, (unsigned)((nrows + kMixRows - 1) / kMixRows), kThreadsMix, msmem, st,
+               reinterpret_cast<float2*>(spec_out), w, bias, nrows, sH);
+    MTD_CHECK_LAUNCH();
+    return launch_cols_blue<true>(reinterpret_cast<const float2*>(spec_out), reinterpret_cast<float2*>(spec_out), nslices,
+                                  H, sH, chirp, bh, st);
+  }
   const size_t smem = (size_t)H * kRSmma * 8 + (size_t)2 * kC2 * kMixLd * 4 + kC2 * 4 + (size_t)H * 8;
 #define CALL(N1_, N2_)                                                                                              \
   {                                                                                                                 \
@@ -655,7 +1004,7 @@ int mtd_fft_cols_mix(const float* spec_in, float* spec_out, const float* w, cons
 int mtd_fft_cols_mix_bwd(const float* spec_x, const float* spec_g, float* spec_out, const float* w, const float* bias,
                          float* part, float* dw, float* db, int B, int H, int W, int C, void* stream) {
   MTD_REQUIRE(spec_x && spec_g && spec_out && w && bias && part && dw && db);
-  MTD_REQUIRE(B > 0 && fft_len_ok(H) && H <= 256 && W >= 2 && C == kC);
+  MTD_REQUIRE(B > 0 && fft_len_ok(H) && H <= 256 && fft_len_ok(W) && C == kC);   // wk below assumes an even W
   const size_t smem = (size_t)H * kRSmma * 16 + kC2 * 4 + (size_t)H * 8;
   const int Wh = W / 2 + 1, nparts = B * Wh;
   cudaStream_t st = (cudaStream_t)stream;

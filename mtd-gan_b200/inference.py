@@ -16,7 +16,8 @@ from . import _ext, ops
 
 
 class GraphedGenerator:
-    """G: ResFFT_Generator in eval mode on a CUDA device.  `micro_batch` slices per graph replay."""
+    """G: ResFFT_Generator in eval mode on a CUDA device; slices of height x width, each from 1 to 512 (512 x 512 is
+    the full CT slice, smaller ones are crops).  `micro_batch` slices per graph replay."""
 
     def __init__(self, G, height: int = 512, width: int = 512, micro_batch: int = 1):
         self.G, self.H, self.W, self.mb = G, int(height), int(width), int(micro_batch)

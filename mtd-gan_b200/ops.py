@@ -763,8 +763,8 @@ class FFTConvBlockFn(Function):
         cfg = _img_cfg(C)
         need_graph = any(ctx.needs_input_grad)
         if _ext.load().mtd_fft_supported(H, W, C) != 1:
-            raise _ext.MtdError(f"FFT_ConvBlock on the B200 path supports 32 channels and H, W in (64, 128, 256, 512); got "
-                                f"C={C}, H={H}, W={W} (the reference's torch.fft.rfft2 takes any size -- not built here)")
+            raise _ext.MtdError(f"FFT_ConvBlock on the B200 path supports 32 channels and 1 <= H, W <= 512; got "
+                                f"C={C}, H={H}, W={W}")
         spec = _empty((_ext.load().mtd_fft_spec_elems(B, H, W, C),), x)
         call("mtd_fft_rows_fwd", fptr(x), fptr(spec), B, H, W, C, st)
         spec2 = _empty(spec.shape, x) if need_graph else spec          # in place when nothing is saved
@@ -789,8 +789,9 @@ class FFTConvBlockFn(Function):
         x, img_w, fft_w, fft_b, spec, img = ctx.saved_tensors
         img_w = ctx.img_w_obj
         B, H, W, C = x.shape
-        if H > 256:
-            raise _ext.MtdError(f"FFT_ConvBlock backward is built for H <= 256 (training patches are 64 x 64); got H={H}")
+        if H not in (64, 128, 256) or W not in (64, 128, 256, 512):
+            raise _ext.MtdError(f"FFT_ConvBlock backward is built for H in (64, 128, 256) and W in (64, 128, 256, 512) "
+                                f"(training patches are 64 x 64); got H={H}, W={W}")
         st = stream()
         cfg = _img_cfg(C)
         need = ctx.needs_input_grad
