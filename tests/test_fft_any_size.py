@@ -1,6 +1,7 @@
 """The Res-FFT-Conv frequency branch at every H, W in [1, 512] (the reference's torch.fft.rfft2 takes any size).
-Lengths 64, 128, 256, 512 run the four-step FFTs (covered by test_gpu_kernels.py / test_gpu_model.py); every other
-length runs the Bluestein kernels.  Checked against torch.fft in fp64 and against the CPU oracle."""
+Lengths 64, 128, 256, 512 run the four-step FFTs; every other length runs the Bluestein kernels.  Checked against
+torch.fft in fp64 and against the CPU oracle.  test_fft_dispatch.py checks that the FFT tests together reach every
+kernel instance of either class."""
 import random
 
 import pytest
@@ -13,7 +14,10 @@ DEV = "cuda"
 gpu = pytest.mark.gpu
 
 ROW_LENGTHS = [1, 2, 7, 37, 63, 65, 96, 100, 255, 384, 500, 509, 511]
-BLOCK_SIZES = [(1, 1), (7, 5), (63, 65), (96, 100), (37, 509), (509, 37), (300, 300), (384, 512), (512, 384), (511, 509)]
+# (128, 128) and (256, 256) run the four-step columns at H = 128 and 256; (64, 7) and (7, 64) mix the four-step and
+# Bluestein classes in one block
+BLOCK_SIZES = [(1, 1), (7, 5), (63, 65), (96, 100), (37, 509), (509, 37), (300, 300), (384, 512), (512, 384), (511, 509),
+               (128, 128), (256, 256), (64, 7), (7, 64)]
 
 
 class Tol:
@@ -155,8 +159,10 @@ def test_out_of_range_and_backward_raise():
     with pytest.raises(_ext.MtdError, match=r"1 <= H, W <= 512"):
         with torch.no_grad():
             blk(torch.zeros(1, 32, 513, 64, device=DEV))
-    x = torch.randn(1, 32, 96, 100, device=DEV, requires_grad=True)
-    out = blk(x)
-    with pytest.raises(_ext.MtdError, match=r"backward is built for"):
-        out.sum().backward()
+    # (512, 64): power-of-two, but the backward kernel's two column slices at H = 512 exceed shared memory
+    for H, W in [(96, 100), (512, 64)]:
+        x = torch.randn(1, 32, H, W, device=DEV, requires_grad=True)
+        out = blk(x)
+        with pytest.raises(_ext.MtdError, match=r"backward is built for"):
+            out.sum().backward()
     torch.cuda.synchronize()

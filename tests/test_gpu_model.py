@@ -90,14 +90,15 @@ def test_generator_forward_512(conv_mode):
     assert rel_err(ob[:1], out) <= 1e-5
 
 
-def test_generator_backward_vs_oracle(conv_mode):
+@pytest.mark.parametrize("B,S", [(2, 64), (1, 128)], ids=["2x64", "1x128"])     # training patches: 64^2, 128^2
+def test_generator_backward_vs_oracle(B, S, conv_mode):
     if conv_mode.mode == "tc1":
         pytest.skip("plain-TF32 opt-in mode: gradients of a 64-layer ReLU net are only sanity-checked at kernel level")
     m = seeded_model()
-    x = O.synthetic_pair(2, 64, seed=41)[0]
+    x = O.synthetic_pair(B, S, seed=41)[0]
     sd = {k: v.detach().cpu().clone().requires_grad_(True) for k, v in m.Generator.state_dict().items()}
     g = torch.Generator().manual_seed(42)
-    w = torch.randn(2, 1, 64, 64, generator=g)
+    w = torch.randn(B, 1, S, S, generator=g)
     (O.generator_forward(sd, x) * w).sum().backward()
     out = m.Generator(x.to(DEV))
     (out * w.to(DEV)).sum().backward()
@@ -105,10 +106,16 @@ def test_generator_backward_vs_oracle(conv_mode):
     sd64 = {k: v.detach().double().requires_grad_(True) for k, v in sd.items()}
     (O.generator_forward(sd64, x.double()) * w.double()).sum().backward()
     tally = GradTally()
+    floors = []
     for k, p in m.Generator.named_parameters():
         floor = rel_err(sd[k].grad, sd64[k].grad)
+        floors.append(floor)
         tally.add(k, rel_err(p.grad, sd[k].grad), max(conv_mode.grad, 30 * floor))
-    tally.finish(conv_mode.median)
+    # where the oracle's own fp32 evaluation misses the mode's median bound (1x128: median fp32-vs-fp64 gap 1.7e-4, more
+    # ReLU units to flip), the bound is twice that gap: the GPU is compared with the fp32 evaluation, two draws of it
+    ref_median = sorted(floors)[len(floors) // 2]
+    print("oracle fp32-vs-fp64 median gap %.2e" % ref_median)
+    tally.finish(conv_mode.median if ref_median <= conv_mode.median else 2 * ref_median)
 
 
 def test_discriminator_vs_golden(masks, conv_mode):
