@@ -157,6 +157,10 @@ int mtd_conv_dgrad_tc(const float* dz, const float* wpd, float* dx, const float*
 int mtd_conv_wgrad_tc_supported(int B, int H, int W, int C1, int C2, int N, int kh, int kw, int stride, int pad);
 int mtd_conv_wgrad_tc(const float* x1, const float* x2, const float* dz, float* gp, int B, int H, int W, int C1, int C2, int N,
                       int kh, int kw, int stride, int pad, int passes, void* stream);
+/* the plan mtd_conv_wgrad_tc runs for these arguments: plan[5] = {1 halo kernel / 0 tap-streaming kernel, Cout tile,
+ * split over pixels, pixel tiles per piece, CTAs}                                                        */
+int mtd_conv_wgrad_tc_plan(int B, int H, int W, int C1, int C2, int N, int kh, int kw, int stride, int pad, int passes,
+                           int* plan);
 /* in place hi <- rna_tf32(w), lo <- rna_tf32(w - hi): operand split for the 3xTF32 mode               */
 int mtd_split_tf32(float* hi, float* lo, long long n, void* stream);
 

@@ -2157,6 +2157,229 @@ bool wg_geometry(int B, int H, int W, int C1, int C2, int N, int kh, int kw, int
   return true;
 }
 
+// ---- weight gradient of a 3x3 / stride-1 / pad-1 layer with an output grid of at least 8 x 8, plain TF32 -----------
+// The tap-streaming kernel above lands every x pixel 9 times (once per tap) per Cout tile, and dz once per 4 units.
+// Here a k-step is one 8 x 8 pixel tile of one image, and a CTA tile is (32-channel chunk cc, BN dz channels, pixel
+// range): per k-step the producer lands three dx-shifted HALO boxes of x — 10 rows x 8 columns, image rows h0-1 .. h0+8,
+// columns w0+dx .. w0+dx+7, zero outside the image — and the BN/32 dz blocks, once for all 9 taps.
+// In the MN-major SW128_32B layout a pixel is one 128 B row, so a box row of 8 pixels is 1024 B: a whole number of
+// swizzle repeats, like the 1024 B k-atom steps (+64 in 16 B units) that every MN-major MMA here already takes.  The dy
+// shift is therefore a pure start-address offset, and the M = 128 operand whose four mn-blocks lie LBO = 1024 B apart is
+// the dx box seen at dy = -1, 0, +1 (+2 is a fourth, unused shift: its rows read the next 1 KB of the stage, which is
+// always landed data, and are never stored).  Three accumulators (dx = -1, 0, +1) of BN columns each.
+// L2 -> SM bytes per k-step: 3 x 10 KB + BN x 256 B for 9 x 32 x BN outputs, against (4 + BN/32) x 8 KB for 4 x 32 x BN
+// on the tap-streaming kernel: 2.3x (BN = 128) to 3.2x (BN = 32) fewer bytes per FLOP.
+constexpr int kHaloPx = 8;                                  // pixel tile edge
+constexpr int kHaloBoxBytes = kHaloPx * (kHaloPx + 2) * 128;  // one dx box: 10 rows x 8 pixels x 32 channels
+
+__host__ __device__ constexpr int wgh_stage_bytes(int bn) { return 3 * kHaloBoxBytes + (bn / 32) * 64 * 128; }
+__host__ __device__ constexpr int wgh_acc_bufs(int bn) { return 6 * bn <= 512 ? 2 : 1; }    // double-buffered if it fits
+
+template <int BN>
+__global__ void __launch_bounds__(kThreads, 1)
+wgrad_halo_kernel(const __grid_constant__ CUtensorMap mapX1, const __grid_constant__ CUtensorMap mapX2,
+                  const __grid_constant__ CUtensorMap mapDz, const __grid_constant__ WgArgs a) {
+  extern __shared__ __align__(1024) unsigned char smem_raw[];
+  constexpr int kBlkBytes = 64 * 128;                           // one 32-channel dz block of the 64-pixel tile
+  constexpr int kNB = BN / 32;
+  constexpr int kStageBytes = wgh_stage_bytes(BN);
+  constexpr int kNAcc = wgh_acc_bufs(BN);
+  constexpr uint32_t kAccCols = 3 * BN;
+  constexpr uint32_t kTmemCols = kNAcc * kAccCols <= 256 ? 256 : 512;
+
+  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  const int S = a.stages;
+  const uint32_t bar_base = base + (uint32_t)S * kStageBytes;
+  auto full_bar = [&](int s) { return bar_base + 8u * s; };
+  auto empty_bar = [&](int s) { return bar_base + 8u * (S + s); };
+  auto conv_bar = [&](int s) { return bar_base + 8u * (2 * S + s); };
+  auto tfull_bar = [&](int i) { return bar_base + 8u * (3 * S + i); };
+  auto tempty_bar = [&](int i) { return bar_base + 8u * (3 * S + 2 + i); };
+  const uint32_t tmem_slot = bar_base + 8u * (3 * S + 4);
+  unsigned char* gen_base = smem_raw + (base - smem_u32(smem_raw));
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int kchunks = a.kc1 + a.kc2;
+  const int Ctot = kchunks * 32;
+
+  if (warp == 0 && lane == 0) {
+    prefetch_tmap(&mapX1);
+    if (a.kc2) prefetch_tmap(&mapX2);
+    prefetch_tmap(&mapDz);
+    for (int s = 0; s < S; ++s) {
+      mbar_init(full_bar(s), 1);
+      mbar_init(empty_bar(s), 1);
+      mbar_init(conv_bar(s), 4);
+    }
+    for (int i = 0; i < kNAcc; ++i) {
+      mbar_init(tfull_bar(i), 1);
+      mbar_init(tempty_bar(i), 4);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(kTmemCols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(gen_base + (tmem_slot - base));
+  mtd_pdl_prologue();
+
+  // tile = ((cc * n_nt) + nt) * ksplit + ks
+  auto decode_tile = [&](int tile, int& cc, int& n0, int& k_begin, int& k_end) {
+    const int ks = tile % a.ksplit;
+    tile /= a.ksplit;
+    k_begin = ks * a.kper;
+    k_end = min(a.ptiles, k_begin + a.kper);
+    n0 = (tile % a.n_nt) * BN;
+    cc = tile / a.n_nt;
+  };
+
+  if (warp == 0) {
+    if (lane == 0) {
+      PipeState st;
+      for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+        int cc, n0, k_begin, k_end;
+        decode_tile(tile, cc, n0, k_begin, k_end);
+        const CUtensorMap* mx = cc < a.kc1 ? &mapX1 : &mapX2;
+        const int c0 = (cc < a.kc1 ? cc : cc - a.kc1) * 32;
+        for (int it = k_begin; it < k_end; ++it) {
+          int pt = it;
+          const int w0 = (pt % a.n_wt) * kHaloPx;
+          pt /= a.n_wt;
+          const int h0 = (pt % a.n_ht) * kHaloPx, b0 = pt / a.n_ht;
+          mbar_wait(empty_bar(st.stage), st.phase ^ 1u);
+          mbar_expect_tx(full_bar(st.stage), (uint32_t)kStageBytes);
+          const uint32_t sa = base + (uint32_t)st.stage * kStageBytes;
+#pragma unroll
+          for (int i = 0; i < 3; ++i) tma_load_4d(mx, sa + i * kHaloBoxBytes, full_bar(st.stage), c0, w0 + i - 1, h0 - 1, b0);
+#pragma unroll
+          for (int j = 0; j < kNB; ++j)
+            tma_load_4d(&mapDz, sa + 3 * kHaloBoxBytes + j * kBlkBytes, full_bar(st.stage), n0 + j * 32, w0, h0, b0);
+          st.advance(S);
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      PipeState st;
+      constexpr uint32_t idesc = make_idesc_mn(BN);
+      int lt = 0;
+      for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x, ++lt) {
+        int cc, n0, k_begin, k_end;
+        decode_tile(tile, cc, n0, k_begin, k_end);
+        const int acc = lt % kNAcc;
+        const uint32_t acc_phase = (uint32_t)(lt / kNAcc) & 1u;
+        mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
+        tc_fence_after();
+        const uint32_t tmem_d = tmem_base + (uint32_t)(acc * kAccCols);
+        for (int it = k_begin; it < k_end; ++it) {
+          mbar_wait(conv_bar(st.stage), st.phase);
+          tc_fence_after();
+          const uint32_t sa = base + (uint32_t)st.stage * kStageBytes;
+          const uint64_t db = make_sw128_desc_mn(sa + 3 * kHaloBoxBytes, kBlkBytes);
+#pragma unroll
+          for (int i = 0; i < 3; ++i) {
+            const uint64_t da = make_sw128_desc_mn(sa + i * kHaloBoxBytes, kHaloPx * 128);     // mn-block j = dy + 1
+#pragma unroll
+            for (int kk = 0; kk < 8; ++kk)
+              umma_tf32(tmem_d + i * BN, da + 64u * kk, db + 64u * kk, idesc, (it > k_begin || kk > 0) ? 1u : 0u);
+          }
+          umma_commit(empty_bar(st.stage));
+          st.advance(S);
+        }
+        umma_commit(tfull_bar(acc));
+      }
+    }
+  } else if (warp < 6) {
+    const int ct = threadIdx.x - 64;
+    PipeState st;
+    for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+      int cc, n0, k_begin, k_end;
+      decode_tile(tile, cc, n0, k_begin, k_end);
+      for (int it = k_begin; it < k_end; ++it) {
+        mbar_wait(full_bar(st.stage), st.phase);
+        float4* tile4 = reinterpret_cast<float4*>(gen_base + (size_t)st.stage * kStageBytes);
+#pragma unroll 4
+        for (int j = 0; j < kStageBytes / 16 / 128; ++j) {
+          float4 v = tile4[ct + 128 * j];
+          uint32_t r0, r1, r2, r3;
+          asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r0) : "f"(v.x));
+          asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r1) : "f"(v.y));
+          asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r2) : "f"(v.z));
+          asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r3) : "f"(v.w));
+          tile4[ct + 128 * j] = make_float4(__uint_as_float(r0), __uint_as_float(r1), __uint_as_float(r2), __uint_as_float(r3));
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncwarp();
+        if (lane == 0) mbar_arrive(conv_bar(st.stage));
+        st.advance(S);
+      }
+    }
+  } else {
+    // TMEM lane quadrant q = accumulator rows 32q .. 32q+31 = mn-block q = tap row dy = q - 1; q = 3 is the unused shift
+    const int q = warp & 3;
+    int lt = 0;
+    for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x, ++lt) {
+      int cc, n0, k_begin, k_end;
+      decode_tile(tile, cc, n0, k_begin, k_end);
+      const int acc = lt % kNAcc;
+      const uint32_t acc_phase = (uint32_t)(lt / kNAcc) & 1u;
+      mbar_wait(tfull_bar(acc), acc_phase);
+      tc_fence_after();
+      if (q < 3) {
+        const int c = cc * 32 + lane;
+#pragma unroll 1
+        for (int i = 0; i < 3; ++i) {
+          const int t = q * 3 + i;
+#pragma unroll 1
+          for (int c0 = 0; c0 < BN; c0 += 32) {
+            uint32_t v[32];
+            tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * kAccCols + i * BN + c0), v);
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+              float* dst = a.gp + ((size_t)(n0 + c0 + j) * 9 + t) * Ctot + c;
+              if (a.ksplit > 1) atomicAdd(dst, __uint_as_float(v[j]));
+              else *dst = __uint_as_float(v[j]);
+            }
+          }
+        }
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(tempty_bar(acc));
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
+  }
+}
+
+template <int BN>
+int launch_wg_halo(const CUtensorMap& mX1, const CUtensorMap& mX2, const CUtensorMap& mDz, WgArgs& a, cudaStream_t st) {
+  constexpr int stage_bytes = wgh_stage_bytes(BN);
+  int stages = (210 * 1024) / stage_bytes;
+  if (stages > 8) stages = 8;
+  if (stages > a.kper) stages = a.kper < 2 ? 2 : a.kper;
+  a.stages = stages;
+  size_t smem = 1024 + (size_t)stages * stage_bytes + 8 * (3 * stages + 4) + 16;
+  static bool attr_set = false;
+  if (!attr_set) {
+    MTD_CUDA(cudaFuncSetAttribute(wgrad_halo_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    attr_set = true;
+  }
+  int grid = a.n_tiles < mtd_sm_count() ? a.n_tiles : mtd_sm_count();
+  mtd_launch(wgrad_halo_kernel<BN>, grid, kThreads, smem, st, mX1, mX2, mDz, a);
+  MTD_CHECK_LAUNCH();
+  return MTD_OK;
+}
+
 __global__ void round_tf32_kernel(float* __restrict__ p, size_t n) {
   mtd_pdl_prologue();
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
@@ -2344,16 +2567,33 @@ int mtd_conv_wgrad_tc_supported(int B, int H, int W, int C1, int C2, int N, int 
   return wg_geometry(B, H, W, C1, C2, N, kh, kw, stride, pad, 64, &tw, &th, &tb) && get_encode() != nullptr ? 1 : 0;
 }
 
-// gp[N][kh*kw][C1+C2] = sum over pixels of dz (x) x on the tensor cores (stride-1 "same" convs).
-int mtd_conv_wgrad_tc(const float* x1, const float* x2, const float* dz, float* gp, int B, int H, int W, int C1, int C2, int N,
-                      int kh, int kw, int stride, int pad, int passes, void* stream) {
-  MTD_REQUIRE(x1 && dz && gp && ((C2 == 0) == (x2 == nullptr)) && (passes == 1 || passes == 3));
-  cudaStream_t st = (cudaStream_t)stream;
-  WgArgs a{};
+// Plan of one weight-gradient call.  Kernel by shape: every 3x3 / stride-1 / pad-1 layer with an output grid of at
+// least 8 x 8 in plain TF32 runs on the halo kernel, everything else on the tap-streaming kernel.  Run alone, the halo
+// kernel is slower than the tap-streaming one at some Cout >= 128 shapes (profiles/r04_wgrad_new_{halo,taps}.txt), but
+// in the train step the weight gradients run on a side stream beside the data gradients, and there its 2.3-3.2x lower
+// L2 traffic and fewer CTAs win: the step is 0.35 ms faster with the halo kernel on every shape it runs than with a
+// per-shape choice of the faster kernel in isolation (profiles/r04_bench_n1_select_*.json).
+// Cout tile BN and split over pixels by a cost model (us):
+//   T = 6 + waves * (2.5 + kper * ts) [+ 3 + 0.33 * ksplit * outputs / 64 K when split]
+// A split adds a memset of the gradient and one fp32 atomic per output element per piece, so layers with few pixels
+// and large weights (the deep discriminator layers) are not split.  ts = one k-step: on the tap-streaming kernel the
+// L2 -> SM time of its stage at ~32 B/clk/SM; on the halo kernel the measured k-step (tools/bench_wgrad.py sweeps,
+// profiles/r04_wgrad_sweep*.txt): 0.95 / 1.2 / 1.7 us at BN = 32 / 64 / 128, bound by its 24 MMAs and shared-memory
+// traffic rather than by L2.  The tap-streaming kernel keeps its widest dz tile (x, its 9x re-read operand, is
+// streamed once per n-tile).  MTD_WG_BN and MTD_WG_KSPLIT force the Cout tile and the split (tuning and test overrides).
+static bool wg_plan(int B, int H, int W, int C1, int C2, int N, int kh, int kw, int stride, int pad, int passes, WgArgs& out,
+                    bool& out_halo, int& out_bn) {
   const int kp = passes == 3 ? 32 : 64;
-  if (!wg_geometry(B, H, W, C1, C2, N, kh, kw, stride, pad, kp, &a.TW, &a.TH, &a.TB)) return MTD_EINVAL;
-  if (!mtd_aligned16(x1) || !mtd_aligned16(dz) || (x2 && !mtd_aligned16(x2))) return MTD_EALIGN;
   const int Ho = (H + 2 * pad - kh) / stride + 1, Wo = (W + 2 * pad - kw) / stride + 1;
+  const bool halo = passes == 1 && kh == 3 && kw == 3 && stride == 1 && pad == 1 && Ho >= kHaloPx && Wo >= kHaloPx;
+  const int forced_bn = getenv("MTD_WG_BN") ? atoi(getenv("MTD_WG_BN")) : 0;
+  const int forced_ks = getenv("MTD_WG_KSPLIT") ? atoi(getenv("MTD_WG_KSPLIT")) : 0;
+  const int sms = mtd_sm_count();
+  double best = 1e30;
+  out_bn = 0;
+  WgArgs a{};
+  if (!wg_geometry(B, H, W, C1, C2, N, kh, kw, stride, pad, kp, &a.TW, &a.TH, &a.TB)) return false;
+  if (halo) { a.TW = a.TH = kHaloPx; a.TB = 1; }
   a.B = B; a.H = Ho; a.W = Wo; a.C1 = C1; a.C2 = C2; a.N = N; a.T = kh * kw; a.es = stride;
   for (int ky = 0; ky < kh; ++ky)
     for (int kx = 0; kx < kw; ++kx) { a.dy[ky * kw + kx] = ky - pad; a.dx[ky * kw + kx] = kx - pad; }
@@ -2361,46 +2601,74 @@ int mtd_conv_wgrad_tc(const float* x1, const float* x2, const float* dz, float* 
   a.ptiles = a.n_wt * a.n_ht * a.n_bt;
   a.kc1 = C1 / 32; a.kc2 = C2 / 32;
   a.units = a.T * (a.kc1 + a.kc2);
-  a.m_tiles = (a.units + 3) / 4;
-  const int sms = mtd_sm_count();
-  // widest dz tile: x (the 9x re-read operand) is streamed once per n-tile; parallelism comes from split-K over pixels
-  int BN = N >= 128 ? 128 : (N >= 64 ? 64 : 32);
-  if (N % BN) return MTD_EINVAL;
-  a.n_nt = N / BN;
-  const int mn = a.m_tiles * a.n_nt;
-  // split over pixels by a cost model (us): a k-step streams 4 units x 64 px x 32 ch of x plus 64 px x BN of dz from L2
-  // (~32 B/clk/SM); every split adds one fp32 atomic per output element (0.33 us per 64 K, measured on the
-  // forward kernel) -- layers with few pixels and large weights (the deep discriminator layers) must NOT be split.
-  int ksplit = 1;
-  {
-    static const int forced = getenv("MTD_WG_KSPLIT") ? atoi(getenv("MTD_WG_KSPLIT")) : 0;     // tuning override
-    const double ts = (128.0 + BN) * kp * 4.0 * (passes == 3 ? 2 : 1) / 61000.0;     // (x rows + dz rows) x pixels x 4 B
-    const double outputs = (double)a.m_tiles * 128.0 * N;
-    double best = 1e30;
-    const int ks_max = a.ptiles / 2 > 1 ? a.ptiles / 2 : 1;
+  a.m_tiles = halo ? a.kc1 + a.kc2 : (a.units + 3) / 4;      // halo: one tile row = one 32-channel chunk, all 9 taps
+  const int ks_max = a.ptiles / 2 > 1 ? a.ptiles / 2 : 1;
+  for (int bn = 128; bn >= 32; bn /= 2) {
+    if (N % bn) continue;
+    if (forced_bn > 0 ? bn != forced_bn : !halo && bn != (N >= 128 ? 128 : N >= 64 ? 64 : 32)) continue;
+    const int mn = a.m_tiles * (N / bn);
+    const double ts = halo ? (bn == 128 ? 1.7 : bn == 64 ? 1.2 : 0.95)
+                           : (128.0 + bn) * kp * 4.0 * (passes == 3 ? 2 : 1) / 61000.0;
+    const double outputs = halo ? (double)a.units * 32.0 * N : (double)a.m_tiles * 128.0 * N;
     for (int ks0 = 1; ks0 <= ks_max && ks0 <= 512; ++ks0) {
       const int kper = (a.ptiles + ks0 - 1) / ks0;
       const int ks = (a.ptiles + kper - 1) / kper;
+      if (forced_ks > 0 && kper != (a.ptiles + min(forced_ks, ks_max) - 1) / min(forced_ks, ks_max)) continue;
       const int waves = (mn * ks + sms - 1) / sms;
       double cost = 6.0 + waves * (2.5 + kper * ts);
       if (ks > 1) cost += 3.0 + 0.33 * ks * outputs / 65536.0;
-      if (cost < best) { best = cost; ksplit = ks; }
+      if (cost < best) {
+        best = cost; out = a; out_halo = halo; out_bn = bn;
+        out.ksplit = ks; out.kper = kper;
+      }
     }
-    if (forced > 0) ksplit = forced < ks_max ? forced : ks_max;
   }
-  a.kper = (a.ptiles + ksplit - 1) / ksplit;
-  ksplit = (a.ptiles + a.kper - 1) / a.kper;
-  a.ksplit = ksplit;
-  a.n_tiles = mn * ksplit;
+  if (!out_bn) return false;
+  out.n_nt = N / out_bn;
+  out.n_tiles = out.m_tiles * out.n_nt * out.ksplit;
+  return true;
+}
+
+// The plan mtd_conv_wgrad_tc runs for these arguments: plan[0] = 1 (halo kernel) / 0 (tap-streaming kernel),
+// plan[1] = Cout tile BN, plan[2] = split over pixels, plan[3] = pixel tiles per piece, plan[4] = CTAs.
+int mtd_conv_wgrad_tc_plan(int B, int H, int W, int C1, int C2, int N, int kh, int kw, int stride, int pad, int passes,
+                           int* plan) {
+  MTD_REQUIRE(plan && (passes == 1 || passes == 3));
+  WgArgs a{};
+  bool halo;
+  int BN;
+  if (!wg_plan(B, H, W, C1, C2, N, kh, kw, stride, pad, passes, a, halo, BN)) return MTD_EINVAL;
+  plan[0] = halo ? 1 : 0; plan[1] = BN; plan[2] = a.ksplit; plan[3] = a.kper;
+  plan[4] = a.n_tiles < mtd_sm_count() ? a.n_tiles : mtd_sm_count();
+  return MTD_OK;
+}
+
+// gp[N][kh*kw][C1+C2] = sum over pixels of dz (x) x on the tensor cores (stride-1 "same" convs).
+int mtd_conv_wgrad_tc(const float* x1, const float* x2, const float* dz, float* gp, int B, int H, int W, int C1, int C2, int N,
+                      int kh, int kw, int stride, int pad, int passes, void* stream) {
+  MTD_REQUIRE(x1 && dz && gp && ((C2 == 0) == (x2 == nullptr)) && (passes == 1 || passes == 3));
+  cudaStream_t st = (cudaStream_t)stream;
+  WgArgs a{};
+  bool halo;
+  int BN;
+  if (!wg_plan(B, H, W, C1, C2, N, kh, kw, stride, pad, passes, a, halo, BN)) return MTD_EINVAL;
+  if (!mtd_aligned16(x1) || !mtd_aligned16(dz) || (x2 && !mtd_aligned16(x2))) return MTD_EALIGN;
   a.gp = gp;
-  if (ksplit > 1) MTD_CUDA(cudaMemsetAsync(gp, 0, (size_t)N * a.T * (C1 + C2) * sizeof(float), st));
+  if (a.ksplit > 1) MTD_CUDA(cudaMemsetAsync(gp, 0, (size_t)N * a.T * (C1 + C2) * sizeof(float), st));
   CUtensorMap mX1, mX2, mDz;
-  int rc = make_act_map(&mX1, x1, C1, W, H, B, a.TW, a.TH, a.TB, true, stride);
+  const int xth = halo ? kHaloPx + 2 : a.TH;                   // halo: 10-row boxes starting one row above the tile
+  int rc = make_act_map(&mX1, x1, C1, W, H, B, a.TW, xth, a.TB, true, stride);
   if (rc) return rc;
-  if (C2) { rc = make_act_map(&mX2, x2, C2, W, H, B, a.TW, a.TH, a.TB, true, stride); if (rc) return rc; }
+  if (C2) { rc = make_act_map(&mX2, x2, C2, W, H, B, a.TW, xth, a.TB, true, stride); if (rc) return rc; }
   else mX2 = mX1;
-  rc = make_act_map(&mDz, dz, N, Wo, Ho, B, a.TW, a.TH, a.TB, true);
+  rc = make_act_map(&mDz, dz, N, a.W, a.H, B, a.TW, a.TH, a.TB, true);
   if (rc) return rc;
+  if (halo) {
+    if (BN == 128) rc = launch_wg_halo<128>(mX1, mX2, mDz, a, st);
+    else if (BN == 64) rc = launch_wg_halo<64>(mX1, mX2, mDz, a, st);
+    else rc = launch_wg_halo<32>(mX1, mX2, mDz, a, st);
+    return rc;
+  }
 #define WG_DISPATCH(BN_) rc = passes == 3 ? launch_wg<BN_, 3, 32>(mX1, mX2, mDz, a, st) : launch_wg<BN_, 1, 64>(mX1, mX2, mDz, a, st)
   if (BN == 128) { WG_DISPATCH(128); }
   else if (BN == 64) { WG_DISPATCH(64); }
